@@ -12,7 +12,11 @@ re-evaluates it, HMC.py:80,82), both Hamiltonians, Metropolis accept, sample boo
 The metric counts S*L grad-evals per step (BASELINE.md §2); `evals_executed_per_step_per_chain` in the
 config is what the library actually ran (L; L+1 in the e2e leg, whose re-uploaded dataset drops the carry).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes, after the timed steps, what the last of them handed its caller (see dump_outputs) as
+DIR/<name>.npy, so that two builds run with the same arguments (hence the same seeded inputs) can be compared output
+for output.
 
 N>1 is launched by torchrun (one rank per GPU).  Chains shard across ranks with no data-path
 collective (weak scaling: 1024 chains per GPU); torch.distributed is used only for the barrier and
@@ -53,7 +57,14 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C1 / C2 / C4 / C5 / strong-scaling sub-records")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0's chains)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 implementation")
+    return args
 
 
 def synth(rows, seed=0):
@@ -61,6 +72,24 @@ def synth(rows, seed=0):
     X = rng.random((rows, D_IN), dtype=np.float32)
     y = rng.integers(0, N_CLS, rows).astype(np.int32)
     return X, y
+
+
+DUMP_STATE_BYTES = 16 << 20           # per state array; the whole dump stays far below 64 MB
+
+
+def dump_outputs(eng, out_dir):
+    """Write what the last HMC step returns to its caller as float32 DIR/<name>.npy: the per-chain energies, log
+    acceptance, decision and loss of that step (hmc_last) and the chains' positions q and momenta p (hmc_state).
+    q and p are chains x parameters (833 MB each at the default config), so only a fixed, seeded set of parameter
+    columns of them is written: every chain, at most DUMP_STATE_BYTES per array."""
+    os.makedirs(out_dir, exist_ok=True)
+    q, p = eng.hmc_state()
+    S, P = q.shape
+    n = max(1, min(P, DUMP_STATE_BYTES // (4 * S)))
+    cols = np.sort(np.random.default_rng(0).choice(P, n, replace=False))
+    arrays = dict(eng.hmc_last(), q_sampled=q[:, cols], p_sampled=p[:, cols])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def measured_peaks():
@@ -461,6 +490,8 @@ def main():
     total_evals = sum_over_ranks(S * L * args.steps)
     value = total_evals / (dev_ms / 1e3)
     accept_rate = d["accept_rate"]
+    if args.dump_outputs and rank == 0:                   # before the e2e leg moves the chains on
+        dump_outputs(eng, args.dump_outputs)
 
     # ---- e2e: same steps through the public C ABI with HOST buffers (H2D of the step's inputs from
     # pinned memory + D2H of the step's result inside the timed region)
