@@ -233,6 +233,10 @@ int pyb_set_option(pyb_handle* h, const char* key, double v) {
   } else if (!strcmp(key, "hmc_carry")) {
     h->opt_hmc_carry = v != 0;
     h->hmc.have_cur = false;
+  } else if (!strcmp(key, "hmc_keep_samples")) {
+    PYB_REQUIRE(!h->hmc.sampling_started, PYB_ERR_STATE,
+                "hmc_keep_samples cannot change during a sampling phase (set it before, or after pyb_hmc_reset_samples)");
+    h->opt_hmc_keep_samples = v != 0;
   } else if (!strcmp(key, "predict_sharded")) {
     h->opt_predict_sharded = v != 0;
   } else if (!strcmp(key, "tc_fuse")) {
@@ -301,6 +305,7 @@ int pyb_get_info(const pyb_handle* h, const char* key, double* out) {
     }
     *out = n ? s / n : 0.0;
   }
+  else if (!strcmp(key, "hmc_arena_rows")) *out = (double)h->hmc.arena_cap;
   else if (!strcmp(key, "i8_guard_ok")) *out = h->i8_guard_ok ? 1.0 : 0.0;
   else if (!strcmp(key, "i8_guard_trips")) *out = (double)h->i8_guard_trips;
   else if (!strcmp(key, "svgd_h")) *out = h->svgd.last_h;
@@ -535,6 +540,7 @@ int pyb_hmc_reset_samples(pyb_handle* h) {
   st.host_samples.clear(); st.host_freq.clear(); st.host_chain.clear();
   st.host_last_idx.assign(st.S, -1);
   st.sampling_started = false;
+  hmc_track_clear(h);
   PYB_CATCH
 }
 
@@ -567,6 +573,41 @@ int pyb_hmc_samples(pyb_handle* h, float* samples, int32_t* freq, int32_t* chain
     if (freq) freq[d] = st.host_freq[i];
     if (chain) chain[d] = st.host_chain[i];
   }
+  PYB_CATCH
+}
+
+int pyb_hmc_track_predictive(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  if (!x) {
+    PYB_CUDA(cudaStreamSynchronize(h->stream));
+    hmc_track_stop(h);
+  } else {
+    hmc_track_start(h, x, Nt, y);
+  }
+  PYB_CATCH
+}
+
+int pyb_hmc_predictive_sums(pyb_handle* h, double* sums_out, double* s2_out, int64_t* n_draws_out) {
+  PYB_TRY
+  PYB_REQUIRE(h && sums_out, PYB_ERR_INVALID, "NULL argument");
+  use_device(h);
+  hmc_track_sums(h, sums_out, s2_out, n_draws_out);
+  PYB_CATCH
+}
+
+int pyb_hmc_predictive_finish(pyb_handle* h, const double* sums, const double* s2, int64_t n_chains, int64_t n_draws,
+                              int32_t uq_semantics, double divisor, float* mean_out, float* var_out, float* rhat_out,
+                              float* total_out, float* aleatoric_out, float* epistemic_out) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  const bool want_uq = total_out || aleatoric_out || epistemic_out;
+  if (want_uq)
+    PYB_REQUIRE(uq_semantics == PYB_UQ_REFERENCE || uq_semantics == PYB_UQ_CANONICAL, PYB_ERR_INVALID, "bad semantics");
+  UncertaintyReq uq{nullptr, uq_semantics == PYB_UQ_REFERENCE ? 1 : 0, divisor, total_out, aleatoric_out, epistemic_out};
+  hmc_track_finish(h, sums, s2, n_chains, n_draws, want_uq ? &uq : nullptr, mean_out, var_out, rhat_out);
   PYB_CATCH
 }
 

@@ -211,7 +211,21 @@ struct HmcState {
   std::vector<float> host_samples;
   std::vector<int32_t> host_freq, host_chain;
   std::vector<int64_t> host_last_idx;   // per chain: index into host arrays of its last sample (-1: none)
-  bool sampling_started = false;
+  bool sampling_started = false;  // a sampling iteration has run since pyb_hmc_init / pyb_hmc_reset_samples
+  // streamed posterior predictive (hmc_predictive.cu): the outputs o of every tracked draw on the tracked inputs
+  struct Track {
+    bool on = false;
+    int64_t Nt = 0, chunk = 0;
+    int64_t T = 0;              // draws per chain so far
+    DevBuf<float> x;            // [Nt, in_dim] library-owned copy of the inputs
+    DevBuf<int32_t> y;          // [Nt] labels (empty: none given)
+    DevBuf<float> out;          // [chunk, Nt, C] forward outputs of one chain chunk
+    DevBuf<float> shift;        // [S, Nt, C] each chain's first tracked draw
+    DevBuf<double> s1c;         // [S, Nt, C] per chain: sum_t (o - shift)
+    DevBuf<double> Q, Qd;       // [Nt, C] pooled sum o^2 and sum (o - shift)^2
+    DevBuf<double> S2;          // [Nt, C, C] pooled sum o o^T (labels given and C > 1)
+    DevBuf<double> part;        // [chain groups, 2, Nt, C] partial sums of one chunk
+  } track;
 };
 
 struct SvgdState {
@@ -321,6 +335,7 @@ struct pyb_handle {
   int opt_fs_cluster = 1;   // 1: the small-width HMC kernel spreads a chain over a CTA cluster when there are few chains
   int opt_live_fused = 1;   // 1: the reference-live SVGD sweep is one cooperative launch on a single GPU
   int opt_hmc_carry = 1;    // 1: loss and gradient at the current position are carried to the next HMC iteration
+  int opt_hmc_keep_samples = 1;   // 1: every tracked HMC draw is recorded (arena + host copy); 0: nothing is kept
   int opt_predict_sharded = 0;   // 1: pyb_predict all-reduces its moment sums over the handle's communicator
   int opt_tc_fuse = 1;   // 1: layer 2 (+ loss, dZ2, dZ1) runs inside the layer-1 GEMM's epilogue where it applies
   int opt_tc_timeline = 0;   // diagnostics: the fused mma kernel records per-CTA cycle sums of its phases (info "tc_timeline_<k>")
@@ -415,6 +430,8 @@ bool tc_supported_rows(pyb_handle* h, int64_t n_rows);
 void tc_eval_batch(pyb_handle* h, const float* Xb, const int32_t* yb_i, const float* yb_f, int64_t Nb, const float* theta,
                    int64_t S, float scale, float* loss_out, float* grad_out);
 void tc_forward(pyb_handle* h, const float* theta, int64_t S, const float* x, int64_t N, float* out);
+void tc_forward_tracked(pyb_handle* h, const float* theta, int64_t S, const float* x, int64_t N, float* out);
+void tc_invalidate_track(pyb_handle* h);
 void gather_rows_f32(pyb_handle* h, const float* src, const int64_t* idx_host, int64_t n, int64_t row_len, float* dst);
 void tc_split_rows(pyb_handle* h, const float* src, int64_t R, int C, int64_t lds, void* hi, void* lo, int64_t ldd);
 void tc_split_transpose(pyb_handle* h, const float* src, int R, int C, int64_t lds, void* hi, void* lo, int64_t ldd);
@@ -476,4 +493,18 @@ struct UncertaintyReq {
 };
 void predict(pyb_handle* h, const float* W, int64_t n, const float* weight, const float* x, int64_t Nt,
              float* mean, float* var, float* all, const UncertaintyReq* uq = nullptr);
+void predictive_finish(pyb_handle* h, const double* s1, const double* s2, const double* S2, double wsum, int64_t Nt,
+                       const int32_t* y_dev, const UncertaintyReq* uq, float* mean, float* var);
+// S2 += sum_k w_k o_k o_k^T over a chunk of outputs [nb, Nt, C] (w NULL: 1)
+void uncert_s2_accum(pyb_handle* h, const float* out, int64_t nb, int64_t Nt, int C, const float* w, double* S2);
+bool is_device_ptr(const void* ptr);
+
+// hmc_predictive.cu
+void hmc_track_start(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y);
+void hmc_track_stop(pyb_handle* h);
+void hmc_track_clear(pyb_handle* h);
+void hmc_track_draw(pyb_handle* h);
+void hmc_track_sums(pyb_handle* h, double* sums, double* s2, int64_t* n_draws);
+void hmc_track_finish(pyb_handle* h, const double* sums, const double* s2, int64_t n_chains, int64_t n_draws,
+                      const UncertaintyReq* uq, float* mean, float* var, float* rhat);
 }  // namespace pyb

@@ -149,6 +149,18 @@ static void launch_uncert_s2(pyb_handle* h, const float* out, int64_t nb, int64_
   constexpr int R = 128 / C;
   k_uncert_s2<C><<<(unsigned)((Nt + R - 1) / R), 128, 0, h->stream>>>(out, nb, Nt, w, S2);
 }
+void uncert_s2_accum(pyb_handle* h, const float* out, int64_t nb, int64_t Nt, int C, const float* w, double* S2) {
+  switch (C) {
+    case 2: launch_uncert_s2<2>(h, out, nb, Nt, w, S2); break;
+    case 3: launch_uncert_s2<3>(h, out, nb, Nt, w, S2); break;
+    case 4: launch_uncert_s2<4>(h, out, nb, Nt, w, S2); break;
+    case 5: launch_uncert_s2<5>(h, out, nb, Nt, w, S2); break;
+    case 10: launch_uncert_s2<10>(h, out, nb, Nt, w, S2); break;
+    default:
+      k_uncert_s2_generic<<<(unsigned)((Nt * C * C + 255) / 256), 256, 0, h->stream>>>(out, nb, Nt, C, w, S2);
+  }
+  count_launch(h);
+}
 // The reference never resets its accumulators between rows (Metrics.py:352-366: `aleatoric +=` inside the row loop,
 // appended per row), so row r of its result is the running sum over rows 0..r.  Three passes over 32-row segments:
 // segment sums, exclusive scan of the segment sums, running prefix written out (fixed order => deterministic).
@@ -189,6 +201,12 @@ __global__ void k_uncert_finish(const double* alea, const double* epi, const dou
   }
 }
 
+bool is_device_ptr(const void* ptr) {
+  cudaPointerAttributes a;
+  if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess) { cudaGetLastError(); return false; }
+  return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+}
+
 // dst[k][:] = src[idx[k]][:]   (device rows of row_len floats; idx arrives from the host)
 __global__ void k_gather_rows_f32(const float* src, const int64_t* idx, int64_t row_len, float* dst) {
   const int64_t k = blockIdx.y;
@@ -210,121 +228,27 @@ void gather_rows_f32(pyb_handle* h, const float* src, const int64_t* idx_host, i
   PYB_CUDA(cudaGetLastError());
 }
 
-void predict(pyb_handle* h, const float* W, int64_t n, const float* weight, const float* x, int64_t Nt,
-             float* mean, float* var, float* all, const UncertaintyReq* uq) {
-  PYB_REQUIRE(n > 0 && Nt > 0, PYB_ERR_INVALID, "n and Nt must be > 0");
-  PYB_REQUIRE(W && x && (uq || (mean && var)), PYB_ERR_INVALID, "null pointer");
-  const Model& m = h->model;
-  const int64_t P = m.P, C = m.out_dim, elems = Nt * C;
-  DevBuf<float> dW, dx, dw, dout, dmean, dvar;
-  DevBuf<double> s1, s2;
-  // classification-uncertainty accumulators [Nt, Ce, Ce] (Ce = 2 for a one-unit output)
+// The finishing tail shared by predict() and the streamed HMC predictive (hmc_predictive.cu): mean / population variance
+// and, with uq, the classification-uncertainty matrices from the moment sums over the draws — s1 = sum w o, s2 = sum w o^2,
+// S2 = sum w o o^T (device [Nt, C, C], C > 1 only), total weight wsum, labels y_dev on the device.  Outputs are host
+// pointers (mean / var may be NULL); ends with a stream synchronisation and last_device_ms measured from ev0.
+void predictive_finish(pyb_handle* h, const double* s1, const double* s2, const double* S2, double wsum, int64_t Nt,
+                       const int32_t* y_dev, const UncertaintyReq* uq, float* mean, float* var) {
+  const int64_t C = h->model.out_dim, elems = Nt * C;
   const int Ce = (C == 1) ? 2 : (int)C, CC = Ce * Ce;
-  DevBuf<double> ua, ue, uS2, seg_a, seg_e, exc_a, exc_e;
-  DevBuf<float> ut, uao, ueo;
-  DevBuf<int32_t> uy;
   const int64_t nseg = (Nt + kUqSeg - 1) / kUqSeg;
+  DevBuf<float> dmean, dvar;
+  DevBuf<double> ua, ue, seg_a, seg_e, exc_a, exc_e;
+  DevBuf<float> ut, uao, ueo;
+  dmean.alloc(elems); dvar.alloc(elems);
   if (uq) {
-    PYB_REQUIRE(uq->y && uq->total && uq->aleatoric && uq->epistemic, PYB_ERR_INVALID, "null pointer");
-    PYB_REQUIRE(CC <= 1024, PYB_ERR_UNSUPPORTED, "classification uncertainty supports at most 32 classes");
-    PYB_REQUIRE(uq->divisor != 0.0, PYB_ERR_INVALID, "divisor must not be 0");
-    for (int64_t r = 0; r < Nt; ++r)
-      PYB_REQUIRE(uq->y[r] >= 0 && uq->y[r] < Ce, PYB_ERR_INVALID, "label out of range");
     ua.alloc(Nt * CC); ue.alloc(Nt * CC); seg_a.alloc(nseg * CC); seg_e.alloc(nseg * CC); exc_a.alloc(nseg * CC); exc_e.alloc(nseg * CC);
-    ut.alloc(Nt * CC); uao.alloc(Nt * CC); ueo.alloc(Nt * CC); uy.alloc(Nt);
-    if (C > 1) {
-      uS2.alloc(Nt * CC);
-      PYB_CUDA(cudaMemsetAsync(uS2.p, 0, Nt * CC * sizeof(double), h->stream));
-    }
-    PYB_CUDA(cudaMemcpyAsync(uy.p, uq->y, Nt * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    ut.alloc(Nt * CC); uao.alloc(Nt * CC); ueo.alloc(Nt * CC);
   }
-  // W and x may be host pointers (copied chunk by chunk) or device pointers (used in place: samples that already
-  // live in HBM, e.g. DLPack tensors, skip the n*P*4-byte upload that otherwise dominates the call)
-  auto on_device = [](const void* ptr) {
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess) { cudaGetLastError(); return false; }
-    return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-  };
-  const bool W_dev = on_device(W), x_dev = on_device(x);
-  // caller-owned device memory (DLPack tensors) was produced on the CALLER's stream; this library works on its own
-  // non-blocking stream, which is ordered against nothing else: wait for the device before reading (header: "device pointers")
-  if (W_dev || x_dev) PYB_CUDA(cudaDeviceSynchronize());
-  const float* xd = x;
-  if (!x_dev) {
-    dx.alloc(Nt * m.in_dim);
-    PYB_CUDA(cudaMemcpyAsync(dx.p, x, Nt * m.in_dim * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    xd = dx.p;
-  }
-  double wsum = 0.0;
-  if (weight) {
-    for (int64_t i = 0; i < n; ++i) wsum += weight[i];
-    dw.alloc(n);
-    PYB_CUDA(cudaMemcpyAsync(dw.p, weight, n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-  } else {
-    wsum = (double)n;
-  }
-  PYB_REQUIRE(wsum > 0.0, PYB_ERR_INVALID, "weights must sum to a positive value");
-  // chunk of samples per pass: bounded by the generic workspace and a 512 MiB output buffer
-  int64_t chunk = generic_chain_batch(h, n, Nt, false);
-  int64_t out_cap = (int64_t)((512ull << 20) / (sizeof(float) * (size_t)elems));
-  if (out_cap < 1) out_cap = 1;
-  chunk = std::min(chunk, out_cap);
-  if (!W_dev) dW.alloc(chunk * P);
-  dout.alloc(chunk * elems);
-  s1.alloc(elems); s2.alloc(elems); dmean.alloc(elems); dvar.alloc(elems);
-  PYB_CUDA(cudaMemsetAsync(s1.p, 0, elems * sizeof(double), h->stream));
-  PYB_CUDA(cudaMemsetAsync(s2.p, 0, elems * sizeof(double), h->stream));
-  const bool use_tensor = tc_supported_rows(h, Nt) && (h->opt_path == PYB_PATH_AUTO || h->opt_path == PYB_PATH_TENSOR);
-  h->path_used = use_tensor ? PYB_PATH_TENSOR : PYB_PATH_GENERIC;
-  PYB_CUDA(cudaEventRecord(h->ev0, h->stream));
-  for (int64_t i0 = 0; i0 < n; i0 += chunk) {
-    int64_t nb = std::min(chunk, n - i0);
-    const float* Wd = W + i0 * P;
-    if (!W_dev) {
-      PYB_CUDA(cudaMemcpyAsync(dW.p, W + i0 * P, nb * P * sizeof(float), cudaMemcpyHostToDevice, h->stream));
-      Wd = dW.p;
-    }
-    if (use_tensor) tc_forward(h, Wd, nb, xd, Nt, dout.p);
-    else generic_forward(h, Wd, nb, xd, Nt, dout.p);
-    k_pred_accum<<<(unsigned)((elems + 255) / 256), 256, 0, h->stream>>>(dout.p, nb, elems, weight ? dw.p + i0 : nullptr,
-                                                                         s1.p, s2.p);
-    count_launch(h);
-    if (uq && C > 1) {
-      const float* wk = weight ? dw.p + i0 : nullptr;
-      switch ((int)C) {
-        case 2: launch_uncert_s2<2>(h, dout.p, nb, Nt, wk, uS2.p); break;
-        case 3: launch_uncert_s2<3>(h, dout.p, nb, Nt, wk, uS2.p); break;
-        case 4: launch_uncert_s2<4>(h, dout.p, nb, Nt, wk, uS2.p); break;
-        case 5: launch_uncert_s2<5>(h, dout.p, nb, Nt, wk, uS2.p); break;
-        case 10: launch_uncert_s2<10>(h, dout.p, nb, Nt, wk, uS2.p); break;
-        default:
-          k_uncert_s2_generic<<<(unsigned)((Nt * CC + 255) / 256), 256, 0, h->stream>>>(dout.p, nb, Nt, (int)C, wk, uS2.p);
-      }
-      count_launch(h);
-    }
-    if (all) {
-      k_nan_to_zero<<<(unsigned)std::min<int64_t>((nb * elems + 255) / 256, 4096), 256, 0, h->stream>>>(dout.p, nb * elems);
-      count_launch(h);
-      PYB_CUDA(cudaMemcpyAsync(all + i0 * elems, dout.p, nb * elems * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    }
-  }
-  // weight samples sharded over ranks (SURVEY 8e): the only exchange is the all-reduce of the moment sums
-  // ([Nt, C] doubles, 0.8 MB each at C5) and of the total weight; per-draw outputs stay with the rank that made them
-  if (h->opt_predict_sharded && h->svgd.nccl_comm && h->svgd.world > 1) {
-    DevBuf<double> dws;
-    dws.alloc(1);
-    PYB_CUDA(cudaMemcpyAsync(dws.p, &wsum, sizeof(double), cudaMemcpyHostToDevice, h->stream));
-    nccl_all_reduce_f64(h->svgd.nccl_comm, s1.p, (size_t)elems, h->stream);
-    nccl_all_reduce_f64(h->svgd.nccl_comm, s2.p, (size_t)elems, h->stream);
-    if (uq && C > 1) nccl_all_reduce_f64(h->svgd.nccl_comm, uS2.p, (size_t)(Nt * CC), h->stream);
-    nccl_all_reduce_f64(h->svgd.nccl_comm, dws.p, 1, h->stream);
-    PYB_CUDA(cudaMemcpyAsync(&wsum, dws.p, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    PYB_CUDA(cudaStreamSynchronize(h->stream));
-  }
-  k_pred_finish<<<(unsigned)((elems + 255) / 256), 256, 0, h->stream>>>(s1.p, s2.p, wsum, elems, dmean.p, dvar.p);
+  k_pred_finish<<<(unsigned)((elems + 255) / 256), 256, 0, h->stream>>>(s1, s2, wsum, elems, dmean.p, dvar.p);
   count_launch(h);
   if (uq) {
-    k_uncert_rows<<<(unsigned)((Nt * CC + 255) / 256), 256, 0, h->stream>>>(s1.p, s2.p, uS2.p, wsum, Nt, (int)C, Ce, uy.p,
+    k_uncert_rows<<<(unsigned)((Nt * CC + 255) / 256), 256, 0, h->stream>>>(s1, s2, S2, wsum, Nt, (int)C, Ce, y_dev,
                                                                            uq->cumulative ? 1 : 0, ua.p, ue.p);
     count_launch(h);
     if (uq->cumulative) {
@@ -351,6 +275,100 @@ void predict(pyb_handle* h, const float* W, int64_t n, const float* weight, cons
   float ms = 0.f;
   PYB_CUDA(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
   h->last_device_ms = ms;
+}
+
+void predict(pyb_handle* h, const float* W, int64_t n, const float* weight, const float* x, int64_t Nt,
+             float* mean, float* var, float* all, const UncertaintyReq* uq) {
+  PYB_REQUIRE(n > 0 && Nt > 0, PYB_ERR_INVALID, "n and Nt must be > 0");
+  PYB_REQUIRE(W && x && (uq || (mean && var)), PYB_ERR_INVALID, "null pointer");
+  const Model& m = h->model;
+  const int64_t P = m.P, C = m.out_dim, elems = Nt * C;
+  DevBuf<float> dW, dx, dw, dout;
+  DevBuf<double> s1, s2;
+  // classification-uncertainty accumulators [Nt, Ce, Ce] (Ce = 2 for a one-unit output)
+  const int Ce = (C == 1) ? 2 : (int)C, CC = Ce * Ce;
+  DevBuf<double> uS2;
+  DevBuf<int32_t> uy;
+  if (uq) {
+    PYB_REQUIRE(uq->y && uq->total && uq->aleatoric && uq->epistemic, PYB_ERR_INVALID, "null pointer");
+    PYB_REQUIRE(CC <= 1024, PYB_ERR_UNSUPPORTED, "classification uncertainty supports at most 32 classes");
+    PYB_REQUIRE(uq->divisor != 0.0, PYB_ERR_INVALID, "divisor must not be 0");
+    for (int64_t r = 0; r < Nt; ++r)
+      PYB_REQUIRE(uq->y[r] >= 0 && uq->y[r] < Ce, PYB_ERR_INVALID, "label out of range");
+    uy.alloc(Nt);
+    if (C > 1) {
+      uS2.alloc(Nt * CC);
+      PYB_CUDA(cudaMemsetAsync(uS2.p, 0, Nt * CC * sizeof(double), h->stream));
+    }
+    PYB_CUDA(cudaMemcpyAsync(uy.p, uq->y, Nt * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+  }
+  // W and x may be host pointers (copied chunk by chunk) or device pointers (used in place: samples that already
+  // live in HBM, e.g. DLPack tensors, skip the n*P*4-byte upload that otherwise dominates the call)
+  const bool W_dev = is_device_ptr(W), x_dev = is_device_ptr(x);
+  // caller-owned device memory (DLPack tensors) was produced on the CALLER's stream; this library works on its own
+  // non-blocking stream, which is ordered against nothing else: wait for the device before reading (header: "device pointers")
+  if (W_dev || x_dev) PYB_CUDA(cudaDeviceSynchronize());
+  const float* xd = x;
+  if (!x_dev) {
+    dx.alloc(Nt * m.in_dim);
+    PYB_CUDA(cudaMemcpyAsync(dx.p, x, Nt * m.in_dim * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    xd = dx.p;
+  }
+  double wsum = 0.0;
+  if (weight) {
+    for (int64_t i = 0; i < n; ++i) wsum += weight[i];
+    dw.alloc(n);
+    PYB_CUDA(cudaMemcpyAsync(dw.p, weight, n * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+  } else {
+    wsum = (double)n;
+  }
+  PYB_REQUIRE(wsum > 0.0, PYB_ERR_INVALID, "weights must sum to a positive value");
+  // chunk of samples per pass: bounded by the generic workspace and a 512 MiB output buffer
+  int64_t chunk = generic_chain_batch(h, n, Nt, false);
+  int64_t out_cap = (int64_t)((512ull << 20) / (sizeof(float) * (size_t)elems));
+  if (out_cap < 1) out_cap = 1;
+  chunk = std::min(chunk, out_cap);
+  if (!W_dev) dW.alloc(chunk * P);
+  dout.alloc(chunk * elems);
+  s1.alloc(elems); s2.alloc(elems);
+  PYB_CUDA(cudaMemsetAsync(s1.p, 0, elems * sizeof(double), h->stream));
+  PYB_CUDA(cudaMemsetAsync(s2.p, 0, elems * sizeof(double), h->stream));
+  const bool use_tensor = tc_supported_rows(h, Nt) && (h->opt_path == PYB_PATH_AUTO || h->opt_path == PYB_PATH_TENSOR);
+  h->path_used = use_tensor ? PYB_PATH_TENSOR : PYB_PATH_GENERIC;
+  PYB_CUDA(cudaEventRecord(h->ev0, h->stream));
+  for (int64_t i0 = 0; i0 < n; i0 += chunk) {
+    int64_t nb = std::min(chunk, n - i0);
+    const float* Wd = W + i0 * P;
+    if (!W_dev) {
+      PYB_CUDA(cudaMemcpyAsync(dW.p, W + i0 * P, nb * P * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+      Wd = dW.p;
+    }
+    if (use_tensor) tc_forward(h, Wd, nb, xd, Nt, dout.p);
+    else generic_forward(h, Wd, nb, xd, Nt, dout.p);
+    k_pred_accum<<<(unsigned)((elems + 255) / 256), 256, 0, h->stream>>>(dout.p, nb, elems, weight ? dw.p + i0 : nullptr,
+                                                                         s1.p, s2.p);
+    count_launch(h);
+    if (uq && C > 1) uncert_s2_accum(h, dout.p, nb, Nt, (int)C, weight ? dw.p + i0 : nullptr, uS2.p);
+    if (all) {
+      k_nan_to_zero<<<(unsigned)std::min<int64_t>((nb * elems + 255) / 256, 4096), 256, 0, h->stream>>>(dout.p, nb * elems);
+      count_launch(h);
+      PYB_CUDA(cudaMemcpyAsync(all + i0 * elems, dout.p, nb * elems * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    }
+  }
+  // weight samples sharded over ranks (SURVEY 8e): the only exchange is the all-reduce of the moment sums
+  // ([Nt, C] doubles, 0.8 MB each at C5) and of the total weight; per-draw outputs stay with the rank that made them
+  if (h->opt_predict_sharded && h->svgd.nccl_comm && h->svgd.world > 1) {
+    DevBuf<double> dws;
+    dws.alloc(1);
+    PYB_CUDA(cudaMemcpyAsync(dws.p, &wsum, sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    nccl_all_reduce_f64(h->svgd.nccl_comm, s1.p, (size_t)elems, h->stream);
+    nccl_all_reduce_f64(h->svgd.nccl_comm, s2.p, (size_t)elems, h->stream);
+    if (uq && C > 1) nccl_all_reduce_f64(h->svgd.nccl_comm, uS2.p, (size_t)(Nt * CC), h->stream);
+    nccl_all_reduce_f64(h->svgd.nccl_comm, dws.p, 1, h->stream);
+    PYB_CUDA(cudaMemcpyAsync(&wsum, dws.p, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    PYB_CUDA(cudaStreamSynchronize(h->stream));
+  }
+  predictive_finish(h, s1.p, s2.p, uS2.p, wsum, Nt, uy.p, uq, mean, var);
 }
 
 }  // namespace pyb

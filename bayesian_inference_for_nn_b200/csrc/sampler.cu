@@ -308,6 +308,7 @@ void hmc_init(pyb_handle* h, int64_t S, int64_t chain_offset, double eps, double
   st.sampling_started = false;
   st.have_inj_p = st.have_inj_u = false;
   st.have_cur = false;
+  hmc_track_stop(h);
   DevBuf<float> tmp;
   const float* q0d = nullptr;
   if (q0) {
@@ -423,12 +424,14 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
   for (int it = 0; it < n_iters; ++it) {
     NvtxRange nv_it("pyb.hmc.iteration");
     bool first = sampling && !st.sampling_started;
-    if (sampling) {
+    const bool record = sampling && h->opt_hmc_keep_samples;   // keep the draws (arena), not only the tracked sums
+    if (record) {
       int64_t need = S * (first ? 2 : 1);
       if (!st.arena.p) hmc_size_arena(h);
       if (st.arena_used_upper + need > st.arena_cap) hmc_flush_arena(h);
       st.arena_used_upper += need;
     }
+    if (first && st.track.on) hmc_track_draw(h);     // the pre-iteration state is the first draw (HMC.py:75-77)
     dim3 gridp = chain_grid(nblk, S);
     if (path == PYB_PATH_FUSED_SMALL) {
       PYB_REQUIRE(fused_small_supported(h), PYB_ERR_UNSUPPORTED, "fused small path does not support this model shape");
@@ -478,18 +481,19 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
     k_accept<<<(unsigned)((S + 255) / 256), 256, 0, h->stream>>>(a);
     count_launch(h);
     }
-    if (sampling) {
+    if (record) {
       k_record_slots<<<1, 1024, 0, h->stream>>>(st.accepted.p, S, first ? 1 : 0, st.arena_count.p, st.arena_freq.p,
                                                 st.arena_chain.p, st.last_idx.p, st.pending_freq.p,
                                                 st.slot_first.p, st.slot_acc.p, st.chain_offset);
       count_launch(h);
-      st.sampling_started = true;
     }
+    if (sampling) st.sampling_started = true;
     const bool carry = h->opt_hmc_carry && path != PYB_PATH_FUSED_SMALL;
     k_select_record<<<gridp, EW_THREADS, 0, h->stream>>>(st.q.p, st.q0.p, st.accepted.p, st.slot_first.p,
-                                                         st.slot_acc.p, st.arena.p, P, sampling ? 1 : 0, S,
+                                                         st.slot_acc.p, st.arena.p, P, record ? 1 : 0, S,
                                                          carry ? st.gcur.p : nullptr, st.g.p);
     count_launch(h);
+    if (sampling && st.track.on) hmc_track_draw(h);  // the post-accept position (HMC.py:92-104)
     if (carry)     // loss at the new current position = what step() returns: accepted ? loss(q_L) : loss(q0) (HMC.py:96,104)
       PYB_CUDA(cudaMemcpyAsync(st.loss0.p, st.ret_loss.p, S * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
     st.have_cur = carry;

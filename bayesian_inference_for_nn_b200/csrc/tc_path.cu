@@ -111,6 +111,7 @@ struct TcData {   // split bf16 operands derived from one [N, D] fp32 matrix res
 };
 struct TcState {
   TcData train, aux;                                    // resident training set / minibatch or test inputs
+  TcData track;                                         // inputs of the streamed HMC predictive (prepared once per tracking)
   int D = 0, H = 0, C = 0;
   int64_t cap_chains = 0, cap_blocks = 0;               // capacity: chains, and 128-row blocks over all chains
   DevBuf<__nv_bfloat16> w_hi, w_lo;                     // W1^T  [chains*H][D]
@@ -145,6 +146,9 @@ int tc_resident_split(const pyb_handle* h) {   // operand split the resident dat
 }
 void tc_invalidate_dataset(pyb_handle* h) {
   if (h->tc) ((TcState*)h->tc)->train.ready = false;
+}
+void tc_invalidate_track(pyb_handle* h) {
+  if (h->tc) ((TcState*)h->tc)->track.ready = false;
 }
 
 // shape conditions of the tensor path for a batch of n_rows data rows
@@ -630,12 +634,8 @@ void tc_eval_batch(pyb_handle* h, const float* Xb, const int32_t* yb_i, const fl
   tc_eval_on(h, st, st->aux, yb_i, yb_f, theta, S, scale, loss_out, grad_out);
 }
 
-// forward only: out [S, N, C] (softmax / output activation applied) for device-resident inputs x [N, D]
-void tc_forward(pyb_handle* h, const float* theta, int64_t S, const float* x, int64_t N, float* out) {
-  TcState* st = tc_state(h);
+static void tc_forward_on(pyb_handle* h, TcState* st, TcData& d, const float* theta, int64_t S, int64_t N, float* out) {
   const Model& m = h->model;
-  tc_prepare_data(h, st->aux, x, N, false);
-  TcData& d = st->aux;
   const int64_t Bc = tc_prepare_bufs(h, st, S, d.Npad, false, d.i8);
   const LayerDesc& L2 = m.layer[1];
   const int64_t P = m.P;
@@ -663,6 +663,23 @@ void tc_forward(pyb_handle* h, const float* theta, int64_t S, const float* x, in
     count_launch(h);
   }
   PYB_CUDA(cudaGetLastError());
+}
+
+// forward only: out [S, N, C] (softmax / output activation applied) for device-resident inputs x [N, D]
+void tc_forward(pyb_handle* h, const float* theta, int64_t S, const float* x, int64_t N, float* out) {
+  TcState* st = tc_state(h);
+  tc_prepare_data(h, st->aux, x, N, false);
+  tc_forward_on(h, st, st->aux, theta, S, N, out);
+}
+
+// the same forward on the tracked inputs of the streamed HMC predictive: their split operands are derived once per
+// tracking (tc_invalidate_track) instead of once per sampling iteration, and the minibatch / test-input set `aux`
+// stays untouched
+void tc_forward_tracked(pyb_handle* h, const float* theta, int64_t S, const float* x, int64_t N, float* out) {
+  TcState* st = tc_state(h);
+  if (!st->track.ready || st->track.N != N || st->track.i8 != i8_mode(h, false, false))
+    tc_prepare_data(h, st->track, x, N, false);
+  tc_forward_on(h, st, st->track, theta, S, N, out);
 }
 
 // ---- building blocks exported to svgd.cu (Gram matrix and Stein contraction on the tensor cores) ----

@@ -115,6 +115,7 @@ class Engine:
         check(self.lib.pyb_hmc_init(self.h, int(S), int(chain_offset), float(eps), float(m), int(L), int(semantics),
                                     _ptr(q0a)))
         self.S = int(S)
+        self._track = None
 
     def hmc_inject(self, p=None, u=None):
         pa = None if p is None else _f32(p, (self.S, self.P))
@@ -162,6 +163,70 @@ class Engine:
         if n:
             check(self.lib.pyb_hmc_samples(self.h, _ptr(s), _ptr(f), _ptr(c)))
         return s, f, c
+
+    # ---- streamed HMC predictive (pyb_hmc_track_predictive / _sums / _finish)
+    def hmc_track_predictive(self, x, y=None):
+        """Accumulate the posterior predictive on inputs x [Nt, in_dim...] (NumPy / DLPack / tf.Tensor, copied once) over
+        every draw the sampler records from the next sampling iteration on; y [Nt] integer labels enable
+        ``hmc_predictive_finish(..., semantics=...)``.  x = None stops tracking."""
+        if x is None:
+            check(self.lib.pyb_hmc_track_predictive(self.h, None, 0, None))
+            self._track = None
+            return
+        if isinstance(x, (np.ndarray, list, tuple)):
+            x = _f32(x)
+            x = x.reshape(x.shape[0], -1)
+        xa, _, xptr = ingest(x, np.float32)
+        if int(np.prod(xa.shape[1:])) != self.spec.in_dim:
+            raise ValueError("x has %d features per row, the model expects %d" % (int(np.prod(xa.shape[1:])), self.spec.in_dim))
+        Nt = int(xa.shape[0])
+        ya = None
+        if y is not None:
+            ya = np.ascontiguousarray(np.asarray(y).reshape(-1), dtype=np.int32)
+            if ya.shape[0] != Nt:
+                raise ValueError("x and y disagree on the number of rows")
+        check(self.lib.pyb_hmc_track_predictive(self.h, xptr, Nt, _ptr(ya)))
+        self._track = (Nt, ya is not None)
+
+    def hmc_predictive_sums(self):
+        """-> (sums [4, Nt, C] float64 = A, Q, M, W; S2 [Nt, C, C] or None; draws per chain T)"""
+        Nt, labels = self._tracked()
+        Cc = self.spec.out_dim
+        sums = np.empty((4, Nt, Cc), np.float64)
+        s2 = np.empty((Nt, Cc, Cc), np.float64) if labels and Cc > 1 else None
+        T = C.c_int64()
+        check(self.lib.pyb_hmc_predictive_sums(self.h, _ptr(sums), _ptr(s2), C.byref(T)))
+        return sums, s2, T.value
+
+    def hmc_predictive_finish(self, sums, s2, n_chains, n_draws, semantics=None, divisor=None):
+        """mean / variance / R-hat [Nt, C] from (summed) ``hmc_predictive_sums``; with ``semantics`` ("reference" |
+        "canonical") also the uncertainty matrices (total, aleatoric, epistemic) [Nt, Ce, Ce] as ``predict_uncertainty``
+        (``divisor`` defaults to the number of rows)."""
+        Nt, _ = self._tracked()
+        Cc = self.spec.out_dim
+        Ce = 2 if Cc == 1 else Cc
+        sums = np.ascontiguousarray(sums, dtype=np.float64)
+        if sums.shape != (4, Nt, Cc):
+            raise ValueError("sums must be [4, %d, %d]" % (Nt, Cc))
+        s2 = None if s2 is None else np.ascontiguousarray(s2, dtype=np.float64)
+        mean, var, rhat = (np.empty((Nt, Cc), np.float32) for _ in range(3))
+        out = dict(mean=mean, variance=var, rhat=rhat)
+        uq = (None, None, None)
+        sem = 0
+        if semantics is not None:
+            sem = {"reference": _lib.UQ_REFERENCE, "canonical": _lib.UQ_CANONICAL}[semantics]
+            uq = tuple(np.empty((Nt, Ce, Ce), np.float32) for _ in range(3))
+            out.update(total=uq[0], aleatoric=uq[1], epistemic=uq[2])
+        check(self.lib.pyb_hmc_predictive_finish(self.h, _ptr(sums), _ptr(s2), int(n_chains), int(n_draws), int(sem),
+                                                 float(Nt if divisor is None else divisor), _ptr(mean), _ptr(var),
+                                                 _ptr(rhat), _ptr(uq[0]), _ptr(uq[1]), _ptr(uq[2])))
+        return out
+
+    def _tracked(self):
+        t = getattr(self, "_track", None)
+        if t is None:
+            raise RuntimeError("no predictive is tracked: call hmc_track_predictive first")
+        return t
 
     # ---- SVGD
     def svgd_init(self, S, lr, semantics=_lib.SVGD_REFERENCE_LIVE, particles0=None, offset=0):

@@ -85,6 +85,25 @@ class EngineGroup:
         parts = self.each(lambda i, e: e.hmc_state())
         return np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts])
 
+    def hmc_track_predictive(self, x, y=None):
+        self.each(lambda i, e: e.hmc_track_predictive(x, y))
+
+    def hmc_predictive(self, semantics=None, divisor=None):
+        """the streamed predictive over every device's chains: the per-device sums are added on the host in device
+        order (they are sums over chains) and finished on engine 0 -> (``hmc_predictive_finish`` dict, n_chains, T)"""
+        parts = self.each(lambda i, e: e.hmc_predictive_sums())
+        Ts = {p[2] for p in parts}
+        if len(Ts) != 1:
+            raise RuntimeError("the devices tracked different numbers of draws per chain: %s" % sorted(Ts))
+        sums, s2 = parts[0][0].copy(), None if parts[0][1] is None else parts[0][1].copy()
+        for p in parts[1:]:
+            sums += p[0]
+            if s2 is not None:
+                s2 += p[1]
+        n_chains = sum(e.S for e in self.engines)
+        T = Ts.pop()
+        return self.engines[0].hmc_predictive_finish(sums, s2, n_chains, T, semantics, divisor), n_chains, T
+
     # ---- SVGD -----------------------------------------------------------------------------------------------------
     def svgd_join(self):
         """one NCCL communicator over the group's engines (a no-op for one device)"""

@@ -15,8 +15,17 @@ Optional knobs (all absent => reference behaviour): ``n_chains``, ``seed`` (abse
 optimizer, kept in ``self.seed``), ``semantics`` ("reference" | "canonical"), ``device``, ``path`` ("auto" | "generic" |
 "fused" | "tensor"), ``chain_offset`` (global id of the first local chain when chains are sharded over processes), and
 ``devices=[0, 1, ...]`` / ``n_devices=k``: the chains are sharded over several GPUs of the box inside this process
-(multi.py) and ``result()`` pools them in global chain order — bit-identical to the one-device run.
+(multi.py) and ``result()`` pools them in global chain order — bit-identical to the one-device run;
+``keep_samples`` (default True): False keeps no sample at all (``result()`` raises) for runs that only need the
+streamed predictive below, whose memory then stays flat however long the chains run.
+
+Streamed predictive: ``track_predictive(x, y=None)`` after ``compile`` and before ``train`` / the first sampling
+``step`` makes every recorded draw go through the forward pass on x while the chains run.  ``predictive()`` then gives
+what ``result().predict(x, 0, mode="exact")`` and ``last_variance`` give, plus the R-hat of every output across the
+chains; ``classification_uncertainty`` what ``result().classification_uncertainty(x, y, 0, mode="exact")`` gives.
 """
+from collections import namedtuple
+
 import numpy as np
 
 from .. import _lib
@@ -24,7 +33,10 @@ from ..distributions import Sampled
 from ..keras_json import parse_model_json
 from ..multi import EngineGroup, devices_from
 from ..nn import BayesianModel
+from ..tensors import to_numpy
 from .Optimizer import Optimizer
+
+Predictive = namedtuple("Predictive", ["mean", "variance", "rhat", "n_chains", "n_draws"])
 
 _PATHS = {"auto": _lib.PATH_AUTO, "generic": _lib.PATH_GENERIC, "fused": _lib.PATH_FUSED_SMALL,
           "tensor": _lib.PATH_TENSOR}
@@ -41,6 +53,9 @@ class HMC(Optimizer):
         self._accepted_runs = 0
         self._current_loss = 0
         self.last_diag = None
+        self._sampling_started = False
+        self._tracking = False
+        self._keep_samples = True
 
     def compile_extra_components(self, **kwargs):
         self._m = self._hyperparameters.m
@@ -60,6 +75,7 @@ class HMC(Optimizer):
         self._devices = devices_from(self._hp)
         self._engine = EngineGroup(self._spec, self._devices, seed=self.seed)
         path = self._hp("path", "auto")
+        self._keep_samples = bool(self._hp("keep_samples", True))
         x, y = self._dataset.training_arrays()          # ONE full-dataset batch, frozen for the run (HMC.py:63-65)
         lowered = prior.lower(self._spec)
 
@@ -67,12 +83,15 @@ class HMC(Optimizer):
             e.set_option("path", _PATHS.get(path, path) if isinstance(path, str) else path)
             e.set_dataset(x, y, self._dataset.loss_kind, n_train=self._dataset.train_size)
             e.set_prior(*lowered)
+            if not self._keep_samples:
+                e.set_option("hmc_keep_samples", 0)
         self._engine.each(setup)
         self._engine.hmc_init(self._n_chains, self._epsilon, self._m, int(self._L), self._semantics,
                               q0=kwargs.get("q0"), chain_offset=int(self._hp("chain_offset", 0)))
 
     # ---- one iteration (HMC.py:74-104) -----------------------------------------------------
     def step(self, save_document_path=None, sampling=True, burning=False):
+        self._sampling_started |= bool(sampling)
         d = self._engine.hmc_run(1, burning=burning, sampling=sampling)
         self._book(d)
         return d["mean_loss"]
@@ -100,6 +119,7 @@ class HMC(Optimizer):
     def train(self, nb_iterations: int, loss_save_document_path: str = None, model_save_frequency: int = None,
               model_save_path: str = None):
         self._accepted_runs = self._total_runs = 0
+        self._sampling_started = True
         self._phase(int(self._nb_burn_epoch), "HMC - Burning", sampling=False, burning=True)
         self._accepted_runs = self._total_runs = 0
         self._engine.each(lambda i, e: e.hmc_reset_samples())
@@ -109,7 +129,41 @@ class HMC(Optimizer):
     def accept_rate(self):
         return self._accepted_runs / max(1, self._total_runs)
 
+    # ---- streamed predictive ---------------------------------------------------------------
+    def track_predictive(self, x, y=None):
+        """Track the posterior predictive on x [Nt, ...] (and, with integer labels y [Nt], the classification
+        uncertainty) over every draw the chains record from here on.  Call after ``compile`` and before ``train`` or the
+        first sampling ``step``."""
+        if self._engine is None:
+            raise RuntimeError("compile the optimizer before tracking the predictive")
+        if self._sampling_started:
+            raise RuntimeError("track_predictive must be called before train() / the first sampling step")
+        self._engine.hmc_track_predictive(to_numpy(x, np.float32), None if y is None else to_numpy(y))
+        self._tracking = True
+
+    def _tracked(self, semantics=None, divisor=None):
+        if not self._tracking:
+            raise RuntimeError("no predictive is tracked: call track_predictive(x) before training")
+        return self._engine.hmc_predictive(semantics, divisor)
+
+    def predictive(self) -> Predictive:
+        """-> (mean, variance, rhat, n_chains, n_draws): the frequency-weighted predictive mean and population variance
+        over every recorded draw, each [Nt, C], and the Gelman-Rubin R-hat of every output across the chains (NaN with
+        fewer than two chains or draws, or where no chain moved)."""
+        r, n_chains, T = self._tracked()
+        return Predictive(r["mean"], r["variance"], r["rhat"], n_chains, T)
+
+    def classification_uncertainty(self, divisor=None, semantics="reference"):
+        """-> (total, aleatoric, epistemic), each [Nt, C, C], over every recorded draw: what
+        ``result().classification_uncertainty(x, y, 0, divisor, semantics, mode="exact")`` returns.  Needs the labels
+        given to ``track_predictive``."""
+        r, _, _ = self._tracked(semantics, divisor)
+        return r["total"], r["aleatoric"], r["epistemic"]
+
     def result(self) -> BayesianModel:
+        if not self._keep_samples:
+            raise RuntimeError("this HMC run keeps no samples (keep_samples=False): use predictive() and "
+                               "classification_uncertainty() for the posterior predictive")
         samples, freq, _chain = self._engine.hmc_samples()
         if samples.shape[0] == 0:
             q, _ = self._engine.hmc_state()          # no sampling iteration yet: current positions, weight 1

@@ -102,9 +102,13 @@ int pyb_param_count(const pyb_handle* h, int64_t* n_params_out);
  * the older kernels that compute the same quantities (used by the tests and by tools/kernel_cycles.sh);
  * "predict_sharded" (default 0, see pyb_set_comm); "hmc_carry" (default 1): the loss and loss gradient at a chain's
  * current position are carried from the previous iteration (its end point if accepted, its start if rejected) instead
- * of being re-evaluated as HMC.py:80,82 do - L instead of L+1 full-data evaluations per iteration, identical results. */
+ * of being re-evaluated as HMC.py:80,82 do - L instead of L+1 full-data evaluations per iteration, identical results;
+ * "hmc_keep_samples" (default 1): every recorded HMC draw is kept for pyb_hmc_samples; 0 keeps none (no sample arena,
+ * no host copy, pyb_hmc_sample_count returns 0) for runs that only need the streamed predictive
+ * (pyb_hmc_track_predictive); the chains move identically either way.  It cannot change during a sampling phase. */
 int pyb_set_option(pyb_handle* h, const char* key, double value);
-/* read-outs: "path_used", "kernel_launches", "last_device_ms", "workspace_bytes", "tensor_path_ok" */
+/* read-outs: "path_used", "kernel_launches", "last_device_ms", "workspace_bytes", "tensor_path_ok", "hmc_arena_rows"
+ * (rows of the device sample arena, 0 while it has never been sized) */
 int pyb_get_info(const pyb_handle* h, const char* key, double* value_out);
 
 /* ---- inputs ---- */
@@ -142,6 +146,34 @@ int pyb_hmc_last(pyb_handle* h, float* U0, float* K0, float* U1, float* K1, floa
 int pyb_hmc_reset_samples(pyb_handle* h);
 int pyb_hmc_sample_count(pyb_handle* h, int64_t* n_out);
 int pyb_hmc_samples(pyb_handle* h, float* samples_out, int32_t* freq_out, int32_t* chain_out);
+
+/* ---- streamed HMC posterior predictive (BayesianModel.predict BayesianModel.py:106-129 in mode "exact" over the draws
+ *      HMC records, HMC.py:92-104; Metrics.classification_uncertainty Metrics.py:344-375) ----
+ * The tracked draws of every chain are exactly the draws pyb_hmc_samples returns with their frequencies: the state
+ * before the first sampling iteration after pyb_hmc_init / pyb_hmc_reset_samples, then the position after every
+ * sampling iteration; burn-in iterations add nothing.  So every chain has the same number T of draws.  Each draw goes
+ * through pyb_predict's forward pass on the tracked inputs (NaN -> 0 per element) inside pyb_hmc_run, on the handle's
+ * stream, and only moment sums are kept.
+ * pyb_hmc_track_predictive: x [Nt, in_dim] float32 host or device (copied once: the caller may free it), y [Nt] int32
+ *   host labels or NULL (needed for the uncertainty matrices; < out_dim, or < 2 for a one-unit output).  Must come before
+ *   the first sampling iteration (PYB_ERR_STATE otherwise); x = NULL stops tracking and frees its memory.  Device memory:
+ *   (8 + 4) S Nt out_dim bytes of per-chain sums, checked up front (PYB_ERR_OOM with the size in the message).
+ *   pyb_hmc_reset_samples clears the sums, pyb_hmc_init stops tracking. */
+int pyb_hmc_track_predictive(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y);
+/* sums_out [4, Nt, out_dim] float64 over this handle's chains: A = sum o, Q = sum o^2, M = sum_s (sum_t o)^2 and
+ * W = sum_s sum_t (o - mean_t o)^2 (the within-chain sum of squares, kept exactly: Q - M/T cancels for chains that
+ * barely move); s2_out [Nt, out_dim, out_dim] = sum o o^T (labels given and out_dim > 1; may be NULL); n_draws_out = T.
+ * All are sums over chains: the sums of handles holding disjoint chains (devices, ranks) add up. */
+int pyb_hmc_predictive_sums(pyb_handle* h, double* sums_out, double* s2_out, int64_t* n_draws_out);
+/* From sums (of this handle, or of several added together) over n_chains chains with n_draws draws each: mean_out /
+ * var_out [Nt, out_dim] as pyb_predict with the samples weighted by their frequencies (population variance);
+ * rhat_out [Nt, out_dim] the Gelman-Rubin R-hat of every output element (classic form, not split or rank-normalised;
+ * NaN when n_chains < 2, n_draws < 2 or the within-chain variance is 0); total / aleatoric / epistemic [Nt, Ce, Ce] as
+ * pyb_predict_uncertainty (uq_semantics, divisor; need the labels and, for out_dim > 1, s2).  Any output may be NULL.
+ * Nt and the labels are this handle's tracked ones. */
+int pyb_hmc_predictive_finish(pyb_handle* h, const double* sums, const double* s2, int64_t n_chains, int64_t n_draws,
+                              int32_t uq_semantics, double divisor, float* mean_out, float* var_out, float* rhat_out,
+                              float* total_out, float* aleatoric_out, float* epistemic_out);
 
 /* ---- SVGD (SVGD.py:219-228 compile, :143-157 init, :84-141 step, :54-68 + :183-202 live kernel,
  *      :165-181 median-heuristic kernel, legacy Adam created :226 applied :120) ---- */
