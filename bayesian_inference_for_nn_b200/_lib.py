@@ -63,6 +63,10 @@ SIGNATURES = {
     "pyb_hmc_reset_samples": [_P],
     "pyb_hmc_sample_count": [_P, C.POINTER(C.c_int64)],
     "pyb_hmc_samples": [_P, _f32p, _i32p, _i32p],
+    "pyb_hmc_adapt_begin": [_P, C.c_double],
+    "pyb_hmc_adapt_end": [_P],
+    "pyb_hmc_step_sizes": [_P, _f64p],
+    "pyb_hmc_set_step_sizes": [_P, _f64p],
     "pyb_hmc_track_predictive": [_P, _f32p, C.c_int64, _i32p],
     "pyb_hmc_predictive_sums": [_P, _f64p, _f64p, C.POINTER(C.c_int64)],
     "pyb_hmc_predictive_finish": [_P, _f64p, _f64p, C.c_int64, C.c_int64, C.c_int32, C.c_double, _f32p, _f32p, _f32p,

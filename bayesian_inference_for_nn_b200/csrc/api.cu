@@ -576,6 +576,38 @@ int pyb_hmc_samples(pyb_handle* h, float* samples, int32_t* freq, int32_t* chain
   PYB_CATCH
 }
 
+int pyb_hmc_adapt_begin(pyb_handle* h, double target_accept) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_adapt_begin(h, target_accept);
+  PYB_CATCH
+}
+
+int pyb_hmc_adapt_end(pyb_handle* h) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_adapt_end(h);
+  PYB_CATCH
+}
+
+int pyb_hmc_step_sizes(pyb_handle* h, double* eps_out) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_step_sizes(h, eps_out);
+  PYB_CATCH
+}
+
+int pyb_hmc_set_step_sizes(pyb_handle* h, const double* eps) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_set_step_sizes(h, eps);
+  PYB_CATCH
+}
+
 int pyb_hmc_track_predictive(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y) {
   PYB_TRY
   PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");

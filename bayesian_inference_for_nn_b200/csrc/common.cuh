@@ -118,6 +118,11 @@ __host__ __device__ inline void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t
   out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
 }
 
+// leapfrog coefficients of a step size e: full kick, half kick, drift (HMC.py:128-141), each computed in double and
+// rounded to float once, so a chain whose own step size equals epsilon gets the scalar path's coefficients bit for bit
+struct StepCoef { float eps, half, drift; };
+__host__ __device__ inline StepCoef step_coef(double e, double m) { return {(float)e, (float)(e / 2), (float)(e / m)}; }
+
 #ifdef __CUDACC__
 // 4 standard normals from one Philox block (two Box-Muller pairs)
 __device__ inline void philox_normal4(uint32_t block, uint32_t chain, uint32_t iter, uint32_t stream,
@@ -161,6 +166,24 @@ __device__ inline T block_sum(T v, T* scratch) {
   T r = (threadIdx.x < nw) ? scratch[threadIdx.x] : T(0);
   if (w == 0) r = warp_sum(r);
   return r;
+}
+
+// Dual averaging of one chain's step size (Hoffman & Gelman 2014, Algorithm 5, with Stan's constants), called from
+// the Metropolis test of every adaptation iteration t = 1, 2, ... (k_accept, k_fs_hmc).  da = {log_eps, log_eps_bar,
+// h_bar, mu}.  The recursion is rounded operation by operation (no contraction into FMAs), as a float64 restatement
+// computes it.
+constexpr double DA_GAMMA = 0.05, DA_T0 = 10.0, DA_KAPPA = 0.75;
+__device__ inline void dual_average(double* da, double* step, float log_alpha, double target, int64_t t) {
+  double a = exp((double)log_alpha);
+  a = (a != a) ? 0.0 : fmin(1.0, a);          // a NaN Hamiltonian difference counts as a rejection
+  const double td = (double)t, eta = 1.0 / (td + DA_T0);
+  const double h_bar = __dadd_rn(__dmul_rn(1.0 - eta, da[2]), __dmul_rn(eta, target - a));
+  const double log_eps = da[3] - __dmul_rn(sqrt(td) / DA_GAMMA, h_bar);
+  const double w = pow(td, -DA_KAPPA);
+  da[0] = log_eps;
+  da[1] = __dadd_rn(__dmul_rn(w, log_eps), __dmul_rn(1.0 - w, da[1]));
+  da[2] = h_bar;
+  *step = exp(log_eps);
 }
 
 __device__ inline float act_apply(float z, int act) {
@@ -212,6 +235,12 @@ struct HmcState {
   std::vector<int32_t> host_freq, host_chain;
   std::vector<int64_t> host_last_idx;   // per chain: index into host arrays of its last sample (-1: none)
   bool sampling_started = false;  // a sampling iteration has run since pyb_hmc_init / pyb_hmc_reset_samples
+  // per-chain step sizes (pyb_hmc_set_step_sizes, pyb_hmc_adapt_begin); unallocated: every chain uses eps
+  DevBuf<double> step;          // [S]
+  DevBuf<double> da;            // [S, 4] dual-averaging state {log_eps, log_eps_bar, h_bar, mu} while adapting
+  bool adapting = false;
+  int64_t adapt_t = 0;          // adaptation iterations run since pyb_hmc_adapt_begin
+  double adapt_target = 0;
   // streamed posterior predictive (hmc_predictive.cu): the outputs o of every tracked draw on the tracked inputs
   struct Track {
     bool on = false;
@@ -446,6 +475,10 @@ void hmc_init(pyb_handle* h, int64_t S, int64_t chain_offset, double eps, double
 void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_diag* out);
 void hmc_eval(pyb_handle* h, const float* q, int64_t S, float* U, float* loss, float* grad);
 void hmc_flush_arena(pyb_handle* h);
+void hmc_adapt_begin(pyb_handle* h, double target);
+void hmc_adapt_end(pyb_handle* h);
+void hmc_step_sizes(pyb_handle* h, double* out);
+void hmc_set_step_sizes(pyb_handle* h, const double* eps);
 
 // svgd.cu
 void svgd_init(pyb_handle* h, int64_t S, int64_t offset, double lr, int sem, const double* p0);

@@ -66,7 +66,10 @@ void fused_small_hmc_iteration(pyb_handle* h, bool burning) {
   p.q = st.q.p; p.p = st.p.p; p.q0 = st.q0.p;
   p.inj_p = st.have_inj_p ? st.inj_p.p : nullptr;
   p.inj_u = st.have_inj_u ? st.inj_u.p : nullptr;
-  p.eps = (float)st.eps; p.half_eps = (float)(st.eps / 2); p.drift = (float)(st.eps / st.m);
+  const StepCoef c = step_coef(st.eps, st.m);
+  p.eps = c.eps; p.half_eps = c.half; p.drift = c.drift;
+  p.step = st.step.p; p.m = st.m;
+  p.da = st.adapting ? st.da.p : nullptr; p.da_target = st.adapt_target; p.da_t = st.adapt_t;
   p.stdv = (st.semantics == PYB_HMC_REFERENCE) ? (float)st.m : (float)sqrt(st.m);
   p.inv2m = (float)(1.0 / (2.0 * st.m));
   p.prior_const = (float)h->prior_const;

@@ -41,6 +41,8 @@ struct FsParams {
   // HMC iteration mode
   float* q; float* p; float* q0; const float* inj_p; const float* inj_u;
   float eps, half_eps, drift, stdv, inv2m, prior_const;
+  double* step; double m;        // step != NULL: per-chain step sizes replace eps / half_eps / drift
+  double* da; double da_target; int64_t da_t;   // da != NULL: adaptation iteration da_t (dual_average)
   int L, semantics, burning;
   int cluster;                   // CTAs per chain (1, 2, 4 or 8)
   uint64_t seed; uint32_t iter; int64_t chain_offset;
@@ -56,6 +58,7 @@ struct FsSmem {
   float* part;    // [n_slices][H*(D+1+C)]
   float* gx;      // [2][GX] cluster exchange: partial gradient [P] + loss sum (double) of this CTA's rows
   double* red;    // [32]
+  float* kc;      // [4] leapfrog coefficients of the chain's step size: full kick, half kick, drift
 };
 
 template <typename T>
@@ -391,6 +394,7 @@ __device__ void fs_setup(const FsParams& p, FsSmem& sm, float* base) {
   float* cur = base;
   const int np = (N + 1) & ~1;
   sm.red = (double*)cur; cur += 64;
+  sm.kc = cur; cur += 4;
   sm.xd = cur; cur += (int64_t)np * (D + C);
   sm.ys = cur; cur += (int64_t)N * (p.loss_kind == PYB_LOSS_SPARSE_CE ? 1 : C);
   sm.qs = cur; cur += P;
@@ -437,6 +441,12 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
   const int64_t s = blockIdx.x / n_ctas, P = p.P;
   const int t = threadIdx.x;
   const bool writer = rank == 0;          // every CTA of the cluster holds the same state; one writes it back
+  // the chain's leapfrog coefficients, kept in shared memory rather than in three registers for the whole kernel; the
+  // per-chain step size is read here, before the writer's Metropolis tail may update it (adaptation)
+  if (t == 0) {
+    const StepCoef c = p.step ? step_coef(p.step[s], p.m) : StepCoef{p.eps, p.half_eps, p.drift};
+    sm.kc[0] = c.eps; sm.kc[1] = c.half; sm.kc[2] = c.drift;
+  }
   int n_eval = 0;
   auto eval = [&]() -> float {
     return n_ctas > 1 ? fs_eval_cluster<D, C, ACT>(p, sm, p.n_train, rank, n_ctas, n_eval) : fs_eval<D, C, ACT>(p, sm, p.n_train);
@@ -460,24 +470,26 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
   // U0 and the first half kick share the evaluation at q0 (HMC.py:80-82)
   const float loss0 = eval();
   double e0 = 0.0;
+  const float half_eps0 = sm.kc[1], drift0 = sm.kc[2];
   for (int64_t i = t; i < P; i += FS_THREADS) {
     float q = sm.qs[i], d = q - p.mu[i], iv = p.inv_var[i];
     e0 += 0.5 * (double)(d * d * iv);
     if (writer) p.q0[s * P + i] = q;
-    float pp = sm.ps[i] - p.half_eps * (sm.gs[i] + d * iv);
+    float pp = sm.ps[i] - half_eps0 * (sm.gs[i] + d * iv);
     sm.ps[i] = pp;
-    sm.qs[i] = q + p.drift * pp;
+    sm.qs[i] = q + drift0 * pp;
   }
   const float Up0 = (float)fs_block_sum_all<double>(e0, sm.red);
   float loss1 = loss0, Up1 = 0.f, K1 = 0.f;
   for (int step = 1; step <= p.L; ++step) {
     loss1 = eval();
+    const float eps = sm.kc[0], half_eps = sm.kc[1], drift = sm.kc[2];
     if (step < p.L) {
       for (int64_t i = t; i < P; i += FS_THREADS) {
         float q = sm.qs[i], d = q - p.mu[i];
-        float pp = sm.ps[i] - p.eps * (sm.gs[i] + d * p.inv_var[i]);
+        float pp = sm.ps[i] - eps * (sm.gs[i] + d * p.inv_var[i]);
         sm.ps[i] = pp;
-        sm.qs[i] = q + p.drift * pp;
+        sm.qs[i] = q + drift * pp;
       }
       __syncthreads();
     } else {
@@ -488,10 +500,10 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
         e1 += 0.5 * (double)(d * d * iv);
         float pp = sm.ps[i];
         if (p.semantics == PYB_HMC_REFERENCE) {   // L-th full kick, then the trailing half kick (HMC.py:85-87)
-          pp = pp - p.eps * gt;
-          pp = pp - p.half_eps * gt;
+          pp = pp - eps * gt;
+          pp = pp - half_eps * gt;
         } else {
-          pp = pp - p.half_eps * gt;
+          pp = pp - half_eps * gt;
         }
         sm.ps[i] = pp;
         k1 += (double)pp * (double)pp;
@@ -515,6 +527,7 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
     float u = p.inj_u ? p.inj_u[s] : philox_uniform((uint32_t)(p.chain_offset + s), p.iter, STREAM_UNIFORM, p.seed);
     int acc = p.burning ? 1 : ((u < alpha) ? 1 : 0);
     p.U0[s] = U0; p.U1[s] = U1; p.K0[s] = K0; p.K1[s] = K1; p.log_alpha[s] = la; p.accepted[s] = acc;
+    if (p.da) dual_average(p.da + 4 * s, p.step + s, la, p.da_target, p.da_t);
     float rl = acc ? loss1 : loss0;
     p.ret_loss[s] = rl;
     if (acc) atomicAdd(&p.counters[0], 1ull);
@@ -530,7 +543,7 @@ static size_t fs_smem_bytes(const pyb_handle* h) {
   const int D = m.layer[0].fan_in, H = m.layer[0].fan_out, C = m.layer[1].fan_out;
   const int n_slices = FS_THREADS / H > 0 ? FS_THREADS / H : 1;
   const size_t np = ((size_t)h->N + 1) & ~(size_t)1;
-  size_t f = 64 + np * D + (size_t)h->N * (h->loss_kind == PYB_LOSS_SPARSE_CE ? 1 : C) + np * C +
+  size_t f = 64 + 4 + np * D + (size_t)h->N * (h->loss_kind == PYB_LOSS_SPARSE_CE ? 1 : C) + np * C +
              3 * (size_t)m.P + (size_t)H * (D + 1 + C) * n_slices + (size_t)H * (((D + 1 + C) + 3) / 4 * 4) + 4 + 2 * (((size_t)m.P + 1) / 2 * 2 + 2) + 2;
   return f * sizeof(float) + 16;
 }

@@ -78,11 +78,25 @@ __global__ void k_finish(const double* partial, int nblk, double scale, float* o
 //                                      separate _step_p calls at q_L, HMC.py:86-87)
 //   [kinetic]  partial_k += p^2                    (HMC.py:161-166)
 //   q += drift*p   (drift==0: skipped)             (HMC.py:138-141)
+// The coefficients are the scalars kick1 / kick2 / drift, or, with per-chain step sizes (step != NULL), those of the
+// block's chain for the leapfrog position `role`.
+enum KickRole {
+  KICK_HALF_DRIFT,   // first half kick + drift (HMC.py:82-83)
+  KICK_FULL_DRIFT,   // full kick + drift (:84-85)
+  KICK_FULL_HALF,    // L-th full kick + trailing half kick, reference semantics (:85-87)
+  KICK_HALF          // trailing half kick, canonical semantics
+};
+__host__ __device__ inline void kick_coefs(int role, const StepCoef& c, float& kick1, float& kick2, float& drift) {
+  kick1 = (role == KICK_HALF_DRIFT || role == KICK_HALF) ? c.half : c.eps;
+  kick2 = role == KICK_FULL_HALF ? c.half : 0.f;
+  drift = (role == KICK_HALF_DRIFT || role == KICK_FULL_DRIFT) ? c.drift : 0.f;
+}
 struct KickArgs {
   float* q; float* p; const float* g; float* q0;
   const float* mu; const float* inv_var;
   int64_t P, S;
   float kick1, kick2, drift;
+  const double* step; double m; int role;
   int snapshot, energy, kinetic;
   double* partial_e; double* partial_k;
 };
@@ -90,6 +104,7 @@ __global__ void __launch_bounds__(EW_THREADS) k_kick_drift(KickArgs a) {
   __shared__ double scratch[32];
   int64_t s = chain_index();
   if (s >= a.S) return;
+  if (a.step) kick_coefs(a.role, step_coef(a.step[s], a.m), a.kick1, a.kick2, a.drift);
   int64_t base = (int64_t)blockIdx.x * EW_CHUNK + threadIdx.x;
   double e = 0.0, k = 0.0;
 #pragma unroll
@@ -157,6 +172,7 @@ struct AcceptArgs {
   int burning;
   float* U0; float* U1; float* log_alpha; int32_t* accepted; float* ret_loss;
   unsigned long long* counters; double* loss_sum;
+  double* da; double* step; double da_target; int64_t da_t;   // da != NULL: adaptation iteration da_t (dual_average)
 };
 __global__ void k_accept(AcceptArgs a) {
   __shared__ double scratch[32];
@@ -172,6 +188,7 @@ __global__ void k_accept(AcceptArgs a) {
     acc = a.burning ? 1 : ((u < alpha) ? 1 : 0);
     isnan_ = (la != la) ? 1 : 0;
     a.U0[s] = U0; a.U1[s] = U1; a.log_alpha[s] = la; a.accepted[s] = acc;
+    if (a.da) dual_average(a.da + 4 * s, a.step + s, la, a.da_target, a.da_t);
     float rl = acc ? a.loss1[s] : a.loss0[s];
     a.ret_loss[s] = rl;
     ls = (double)rl;
@@ -308,6 +325,9 @@ void hmc_init(pyb_handle* h, int64_t S, int64_t chain_offset, double eps, double
   st.sampling_started = false;
   st.have_inj_p = st.have_inj_u = false;
   st.have_cur = false;
+  st.adapting = false;
+  st.adapt_t = 0;
+  st.step.release(); st.da.release();
   hmc_track_stop(h);
   DevBuf<float> tmp;
   const float* q0d = nullptr;
@@ -369,15 +389,16 @@ void hmc_flush_arena(pyb_handle* h) {
   st.arena_used_upper = 0;
 }
 
-static void launch_kick(pyb_handle* h, const float* g, float kick1, float kick2, float drift, bool snapshot, bool energy,
-                        bool kinetic, float* Up_out, float* K_out) {
+static void launch_kick(pyb_handle* h, const float* g, KickRole role, bool snapshot, bool energy, bool kinetic,
+                        float* Up_out, float* K_out) {
   NvtxRange nv("pyb.hmc.kick_drift");
   HmcState& st = h->hmc;
   const int64_t P = h->model.P;
   int nblk = ew_blocks(P);
   KickArgs a;
   a.q = st.q.p; a.p = st.p.p; a.g = g; a.q0 = st.q0.p; a.mu = h->mu.p; a.inv_var = h->inv_var.p; a.P = P; a.S = st.S;
-  a.kick1 = kick1; a.kick2 = kick2; a.drift = drift;
+  kick_coefs(role, step_coef(st.eps, st.m), a.kick1, a.kick2, a.drift);
+  a.step = st.step.p; a.m = st.m; a.role = role;
   a.snapshot = snapshot; a.energy = energy; a.kinetic = kinetic;
   a.partial_e = st.partial_e.p; a.partial_k = st.partial_k.p;
   k_kick_drift<<<chain_grid(nblk, st.S), EW_THREADS, 0, h->stream>>>(a);
@@ -407,10 +428,10 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
   HmcState& st = h->hmc;
   PYB_REQUIRE(st.inited, PYB_ERR_STATE, "pyb_hmc_init must be called first");
   PYB_REQUIRE(n_iters >= 0, PYB_ERR_INVALID, "n_iters must be >= 0");
+  PYB_REQUIRE(!(sampling && st.adapting), PYB_ERR_STATE,
+              "no sampling while the step sizes adapt: call pyb_hmc_adapt_end first");
   const int64_t P = h->model.P, S = st.S;
   const int nblk = ew_blocks(P);
-  const float eps = (float)st.eps;
-  const float half = (float)(st.eps / 2), drift = (float)(st.eps / st.m);
   const float n_train = (float)h->n_train;
   const float stdv = (st.semantics == PYB_HMC_REFERENCE) ? (float)st.m : (float)sqrt(st.m);
   int64_t launches0 = h->kernel_launches;
@@ -432,6 +453,7 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
       st.arena_used_upper += need;
     }
     if (first && st.track.on) hmc_track_draw(h);     // the pre-iteration state is the first draw (HMC.py:75-77)
+    if (st.adapting) st.adapt_t++;
     dim3 gridp = chain_grid(nblk, S);
     if (path == PYB_PATH_FUSED_SMALL) {
       PYB_REQUIRE(fused_small_supported(h), PYB_ERR_UNSUPPORTED, "fused small path does not support this model shape");
@@ -456,17 +478,17 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
       eval_loss_grad(h, st.q.p, S, n_train, st.loss0.p, st.gcur.p);
       evals += S;
     }
-    launch_kick(h, st.gcur.p, half, 0.f, drift, true, true, false, st.Up0.p, nullptr);
+    launch_kick(h, st.gcur.p, KICK_HALF_DRIFT, true, true, false, st.Up0.p, nullptr);
     for (int i = 1; i <= st.L; ++i) {
       eval_loss_grad(h, st.q.p, S, n_train, st.loss.p, st.g.p);
       evals += S;
       if (i < st.L) {
-        launch_kick(h, st.g.p, eps, 0.f, drift, false, false, false, nullptr, nullptr);
+        launch_kick(h, st.g.p, KICK_FULL_DRIFT, false, false, false, nullptr, nullptr);
       } else if (st.semantics == PYB_HMC_REFERENCE) {
         // L-th full kick and the trailing half kick, both with the gradient at q_L (HMC.py:85-87)
-        launch_kick(h, st.g.p, eps, half, 0.f, false, true, true, st.Up1.p, st.K1.p);
+        launch_kick(h, st.g.p, KICK_FULL_HALF, false, true, true, st.Up1.p, st.K1.p);
       } else {
-        launch_kick(h, st.g.p, half, 0.f, 0.f, false, true, true, st.Up1.p, st.K1.p);
+        launch_kick(h, st.g.p, KICK_HALF, false, true, true, st.Up1.p, st.K1.p);
       }
     }
     NvtxRange nv_acc("pyb.hmc.accept");
@@ -478,6 +500,7 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
     a.burning = burning ? 1 : 0;
     a.U0 = st.U0.p; a.U1 = st.U1.p; a.log_alpha = st.log_alpha.p; a.accepted = st.accepted.p;
     a.ret_loss = st.ret_loss.p; a.counters = st.counters.p; a.loss_sum = st.loss_sum.p;
+    a.da = st.adapting ? st.da.p : nullptr; a.step = st.step.p; a.da_target = st.adapt_target; a.da_t = st.adapt_t;
     k_accept<<<(unsigned)((S + 255) / 256), 256, 0, h->stream>>>(a);
     count_launch(h);
     }
@@ -555,6 +578,90 @@ void hmc_eval(pyb_handle* h, const float* q, int64_t S, float* U, float* loss, f
   if (grad) PYB_CUDA(cudaMemcpyAsync(grad, dg.p, S * P * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
   PYB_CUDA(cudaStreamSynchronize(h->stream));
   PYB_CUDA(cudaGetLastError());
+}
+
+// ------------------------------------------------------------------------------------------
+// per-chain step sizes and their dual-averaging adaptation (dual_average, common.cuh)
+// ------------------------------------------------------------------------------------------
+__global__ void k_adapt_begin(const double* step, double* da, int64_t S) {
+  int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= S) return;
+  da[4 * s + 0] = log(step[s]);
+  da[4 * s + 1] = 0.0;
+  da[4 * s + 2] = 0.0;
+  da[4 * s + 3] = log(10.0 * step[s]);      // mu: the adaptation leans towards larger steps than it starts from
+}
+__global__ void k_adapt_end(double* step, const double* da, int64_t S) {
+  int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s < S) step[s] = exp(da[4 * s + 1]);
+}
+
+static void require_inited(const HmcState& st) {
+  PYB_REQUIRE(st.inited, PYB_ERR_STATE, "pyb_hmc_init must be called first");
+}
+
+// the per-chain array, every chain at epsilon, the first time it is needed
+static void ensure_step_array(pyb_handle* h) {
+  HmcState& st = h->hmc;
+  if (st.step.p) return;
+  std::vector<double> e((size_t)st.S, st.eps);
+  st.step.alloc(st.S);
+  PYB_CUDA(cudaMemcpyAsync(st.step.p, e.data(), st.S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
+}
+
+void hmc_adapt_begin(pyb_handle* h, double target) {
+  HmcState& st = h->hmc;
+  require_inited(st);
+  PYB_REQUIRE(!st.adapting, PYB_ERR_STATE, "the step sizes are already adapting");
+  PYB_REQUIRE(target > 0.0 && target < 1.0, PYB_ERR_INVALID, "target_accept must be in (0, 1)");
+  st.da.alloc(4 * st.S);
+  ensure_step_array(h);
+  k_adapt_begin<<<(unsigned)((st.S + 255) / 256), 256, 0, h->stream>>>(st.step.p, st.da.p, st.S);
+  count_launch(h);
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
+  PYB_CUDA(cudaGetLastError());
+  st.adapting = true;
+  st.adapt_t = 0;
+  st.adapt_target = target;
+}
+
+void hmc_adapt_end(pyb_handle* h) {
+  HmcState& st = h->hmc;
+  require_inited(st);
+  PYB_REQUIRE(st.adapting, PYB_ERR_STATE, "the step sizes are not adapting: call pyb_hmc_adapt_begin first");
+  if (st.adapt_t > 0) {        // without an adaptation iteration the step sizes stay where they started
+    k_adapt_end<<<(unsigned)((st.S + 255) / 256), 256, 0, h->stream>>>(st.step.p, st.da.p, st.S);
+    count_launch(h);
+  }
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
+  PYB_CUDA(cudaGetLastError());
+  st.adapting = false;
+  st.da.release();
+}
+
+void hmc_step_sizes(pyb_handle* h, double* out) {
+  HmcState& st = h->hmc;
+  require_inited(st);
+  PYB_REQUIRE(out, PYB_ERR_INVALID, "NULL argument");
+  if (!st.step.p) {
+    std::fill(out, out + st.S, st.eps);
+    return;
+  }
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
+  PYB_CUDA(cudaMemcpy(out, st.step.p, st.S * sizeof(double), cudaMemcpyDeviceToHost));
+}
+
+void hmc_set_step_sizes(pyb_handle* h, const double* eps) {
+  HmcState& st = h->hmc;
+  require_inited(st);
+  PYB_REQUIRE(!st.adapting, PYB_ERR_STATE, "the step sizes are adapting: call pyb_hmc_adapt_end first");
+  PYB_REQUIRE(eps, PYB_ERR_INVALID, "NULL argument");
+  for (int64_t s = 0; s < st.S; ++s)
+    PYB_REQUIRE(isfinite(eps[s]) && eps[s] > 0.0, PYB_ERR_INVALID, "step sizes must be finite and > 0");
+  st.step.alloc(st.S);
+  PYB_CUDA(cudaMemcpyAsync(st.step.p, eps, st.S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
 }
 
 }  // namespace pyb

@@ -164,6 +164,29 @@ class Engine:
             check(self.lib.pyb_hmc_samples(self.h, _ptr(s), _ptr(f), _ptr(c)))
         return s, f, c
 
+    # ---- per-chain step sizes (pyb_hmc_adapt_begin / _end, pyb_hmc_step_sizes, pyb_hmc_set_step_sizes)
+    def hmc_adapt_begin(self, target=0.8):
+        """From the next ``hmc_run`` on, adapt every chain's step size by dual averaging towards the acceptance
+        probability ``target`` (0 < target < 1); no sampling iteration until ``hmc_adapt_end``."""
+        check(self.lib.pyb_hmc_adapt_begin(self.h, float(target)))
+
+    def hmc_adapt_end(self):
+        """Freeze every chain's step size at its dual-averaging mean."""
+        check(self.lib.pyb_hmc_adapt_end(self.h))
+
+    def hmc_step_sizes(self):
+        """-> [S] float64: each chain's step size (epsilon for all while none was set or adapted)."""
+        out = np.empty(self.S, np.float64)
+        check(self.lib.pyb_hmc_step_sizes(self.h, _ptr(out)))
+        return out
+
+    def hmc_set_step_sizes(self, eps):
+        """eps [S]: one step size per chain, each finite and > 0."""
+        e = np.ascontiguousarray(eps, dtype=np.float64).reshape(-1)
+        if e.shape[0] != self.S:
+            raise ValueError("expected %d step sizes, got %d" % (self.S, e.shape[0]))
+        check(self.lib.pyb_hmc_set_step_sizes(self.h, _ptr(e)))
+
     # ---- streamed HMC predictive (pyb_hmc_track_predictive / _sums / _finish)
     def hmc_track_predictive(self, x, y=None):
         """Accumulate the posterior predictive on inputs x [Nt, in_dim...] (NumPy / DLPack / tf.Tensor, copied once) over

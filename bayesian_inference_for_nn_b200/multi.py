@@ -85,6 +85,22 @@ class EngineGroup:
         parts = self.each(lambda i, e: e.hmc_state())
         return np.concatenate([p[0] for p in parts]), np.concatenate([p[1] for p in parts])
 
+    def hmc_adapt_begin(self, target):
+        self.each(lambda i, e: e.hmc_adapt_begin(target))     # chains adapt on their own: no cross-device step
+
+    def hmc_adapt_end(self):
+        self.each(lambda i, e: e.hmc_adapt_end())
+
+    def hmc_step_sizes(self):
+        """[n_chains] float64 in global chain order"""
+        return np.concatenate(self.each(lambda i, e: e.hmc_step_sizes()))
+
+    def hmc_set_step_sizes(self, eps):
+        eps = np.asarray(eps, np.float64).reshape(-1)
+        if eps.shape[0] != self.ranges[-1][1]:
+            raise ValueError("expected %d step sizes, got %d" % (self.ranges[-1][1], eps.shape[0]))
+        self.each(lambda i, e: e.hmc_set_step_sizes(eps[self.ranges[i][0]:self.ranges[i][1]]))
+
     def hmc_track_predictive(self, x, y=None):
         self.each(lambda i, e: e.hmc_track_predictive(x, y))
 

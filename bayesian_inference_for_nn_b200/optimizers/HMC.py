@@ -19,6 +19,15 @@ optimizer, kept in ``self.seed``), ``semantics`` ("reference" | "canonical"), ``
 ``keep_samples`` (default True): False keeps no sample at all (``result()`` raises) for runs that only need the
 streamed predictive below, whose memory then stays flat however long the chains run.
 
+Step-size adaptation: ``adapt_iterations`` (default 0: off) and ``target_accept`` (default 0.8).  With
+``adapt_iterations = n > 0``, ``train(k)`` runs the reference's burn-in unchanged, then n iterations (progress line
+"HMC - Adapting") in which every chain tunes its own step size by dual averaging (Hoffman & Gelman 2014, Algorithm 5;
+Stan's constants) towards an average acceptance probability of ``target_accept``, starting from ``epsilon``; then the
+step sizes are frozen and the k sampling iterations run as before.  Adaptation draws nothing into the samples, and
+``accept_rate`` still covers the sampling iterations only.  ``step_sizes`` gives every chain's step size ([n_chains]
+float64, global chain order; ``epsilon`` everywhere without adaptation).  Chains adapt independently, so a run sharded
+over devices gives the one-device step sizes.
+
 Streamed predictive: ``track_predictive(x, y=None)`` after ``compile`` and before ``train`` / the first sampling
 ``step`` makes every recorded draw go through the forward pass on x while the chains run.  ``predictive()`` then gives
 what ``result().predict(x, 0, mode="exact")`` and ``last_variance`` give, plus the R-hat of every output across the
@@ -56,6 +65,8 @@ class HMC(Optimizer):
         self._sampling_started = False
         self._tracking = False
         self._keep_samples = True
+        self._adapt_iterations = 0
+        self._target_accept = 0.8
 
     def compile_extra_components(self, **kwargs):
         self._m = self._hyperparameters.m
@@ -72,6 +83,12 @@ class HMC(Optimizer):
         # explicit seed every optimizer draws its own, so repeated runs are independent; self.seed reproduces a run
         seed = self._hp("seed", None)
         self.seed = int(np.random.SeedSequence().entropy & ((1 << 63) - 1)) if seed is None else int(seed)
+        self._adapt_iterations = int(self._hp("adapt_iterations", 0))
+        self._target_accept = float(self._hp("target_accept", 0.8))
+        if self._adapt_iterations < 0:
+            raise ValueError("adapt_iterations must be >= 0")
+        if not 0.0 < self._target_accept < 1.0:
+            raise ValueError("target_accept must be in (0, 1)")
         self._devices = devices_from(self._hp)
         self._engine = EngineGroup(self._spec, self._devices, seed=self.seed)
         path = self._hp("path", "auto")
@@ -121,6 +138,11 @@ class HMC(Optimizer):
         self._accepted_runs = self._total_runs = 0
         self._sampling_started = True
         self._phase(int(self._nb_burn_epoch), "HMC - Burning", sampling=False, burning=True)
+        if self._adapt_iterations > 0:
+            self._accepted_runs = self._total_runs = 0
+            self._engine.hmc_adapt_begin(self._target_accept)
+            self._phase(self._adapt_iterations, "HMC - Adapting", sampling=False, burning=False)
+            self._engine.hmc_adapt_end()
         self._accepted_runs = self._total_runs = 0
         self._engine.each(lambda i, e: e.hmc_reset_samples())
         self._phase(int(nb_iterations), "HMC - Sampling", sampling=True, burning=False)
@@ -128,6 +150,11 @@ class HMC(Optimizer):
     @property
     def accept_rate(self):
         return self._accepted_runs / max(1, self._total_runs)
+
+    @property
+    def step_sizes(self):
+        """[n_chains] float64: every chain's step size, in global chain order"""
+        return self._engine.hmc_step_sizes()
 
     # ---- streamed predictive ---------------------------------------------------------------
     def track_predictive(self, x, y=None):

@@ -147,6 +147,29 @@ int pyb_hmc_reset_samples(pyb_handle* h);
 int pyb_hmc_sample_count(pyb_handle* h, int64_t* n_out);
 int pyb_hmc_samples(pyb_handle* h, float* samples_out, int32_t* freq_out, int32_t* chain_out);
 
+/* ---- per-chain step sizes and their adaptation (the reference uses one epsilon for its one chain, HMC.py:53-55) ----
+ * Every chain may have its own step size e_s; its leapfrog then kicks by (float)e_s and (float)(e_s/2) and drifts by
+ * (float)(e_s/m), each rounded once from double, so a chain whose e_s equals epsilon moves exactly as with the scalar.
+ * Until step sizes are set or adapted, every chain uses epsilon.  pyb_hmc_init ends any adaptation and drops the
+ * per-chain step sizes.  Before pyb_hmc_init all four calls return PYB_ERR_STATE.
+ * pyb_hmc_adapt_begin: from the next pyb_hmc_run on, every iteration (burn-in included) updates each chain's step size
+ *   by dual averaging (Hoffman & Gelman 2014, Algorithm 5) towards an acceptance probability of target_accept
+ *   (0 < target < 1, else PYB_ERR_INVALID; PYB_ERR_STATE if already adapting).  Per chain and adaptation iteration
+ *   t = 1, 2, ... with a = min(1, exp(log_alpha)) (NaN: 0), gamma = 0.05, t0 = 10, kappa = 0.75 (Stan's defaults):
+ *     h_bar = (1 - 1/(t + t0)) h_bar + (target - a)/(t + t0);  log_eps = mu - sqrt(t)/gamma h_bar;
+ *     log_eps_bar = t^-kappa log_eps + (1 - t^-kappa) log_eps_bar;  e_s = exp(log_eps)
+ *   starting from mu = log(10 e_s), h_bar = 0, log_eps_bar = 0.  Chains adapt independently: a sharded run adapts as
+ *   the unsharded one.  While adapting, pyb_hmc_run with sampling = 1 returns PYB_ERR_STATE (draws taken while the
+ *   step sizes move are not draws from the posterior).
+ * pyb_hmc_adapt_end: freezes e_s = exp(log_eps_bar) (unchanged if no iteration ran); PYB_ERR_STATE if not adapting.
+ * pyb_hmc_step_sizes: eps_out [S] host float64, the current e_s (epsilon for every chain when never set or adapted).
+ * pyb_hmc_set_step_sizes: eps [S] host float64, each finite and > 0 (else PYB_ERR_INVALID); PYB_ERR_STATE while
+ *   adapting. */
+int pyb_hmc_adapt_begin(pyb_handle* h, double target_accept);
+int pyb_hmc_adapt_end(pyb_handle* h);
+int pyb_hmc_step_sizes(pyb_handle* h, double* eps_out);
+int pyb_hmc_set_step_sizes(pyb_handle* h, const double* eps);
+
 /* ---- streamed HMC posterior predictive (BayesianModel.predict BayesianModel.py:106-129 in mode "exact" over the draws
  *      HMC records, HMC.py:92-104; Metrics.classification_uncertainty Metrics.py:344-375) ----
  * The tracked draws of every chain are exactly the draws pyb_hmc_samples returns with their frequencies: the state
