@@ -281,6 +281,7 @@ int pyb_get_info(const pyb_handle* h, const char* key, double* out) {
   else if (!strcmp(key, "kernel_launches")) *out = (double)h->kernel_launches;
   else if (!strcmp(key, "last_device_ms")) *out = h->last_device_ms;
   else if (!strcmp(key, "sm_count")) *out = h->sm_count;
+  else if (!strcmp(key, "fs_cluster_used")) *out = h->fs_cluster_used;
   else if (!strcmp(key, "prof_ms")) *out = h->prof_ms;
   else if (!strcmp(key, "prof_flops")) *out = h->prof_flops;
   else if (!strcmp(key, "prof_launches")) *out = (double)h->prof_launches;

@@ -390,6 +390,7 @@ struct pyb_handle {
   double opt_workspace_mb = 4096;
   int64_t opt_chain_batch = 0;
   int path_used = PYB_PATH_GENERIC;
+  int fs_cluster_used = 0;  // CTAs per chain of the last small-width HMC launch (0 before the first)
   int64_t kernel_launches = 0;
   double last_device_ms = 0;
   pyb::Workspace ws;

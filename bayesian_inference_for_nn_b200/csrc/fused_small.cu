@@ -80,6 +80,7 @@ void fused_small_hmc_iteration(pyb_handle* h, bool burning) {
   if (h->opt_fs_cluster)
     for (int c = 8; c >= 2; c >>= 1)
       if (st.S * c <= h->sm_count && h->N / c >= 64) { p.cluster = c; break; }
+  h->fs_cluster_used = p.cluster;
   p.U0 = st.U0.p; p.U1 = st.U1.p; p.K0 = st.K0.p; p.K1 = st.K1.p; p.log_alpha = st.log_alpha.p;
   p.ret_loss = st.ret_loss.p; p.accepted = st.accepted.p; p.counters = st.counters.p; p.loss_sum = st.loss_sum.p;
   fs_dispatch(h, p, st.S, true);

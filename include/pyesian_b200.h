@@ -108,7 +108,8 @@ int pyb_param_count(const pyb_handle* h, int64_t* n_params_out);
  * (pyb_hmc_track_predictive); the chains move identically either way.  It cannot change during a sampling phase. */
 int pyb_set_option(pyb_handle* h, const char* key, double value);
 /* read-outs: "path_used", "kernel_launches", "last_device_ms", "workspace_bytes", "tensor_path_ok", "hmc_arena_rows"
- * (rows of the device sample arena, 0 while it has never been sized) */
+ * (rows of the device sample arena, 0 while it has never been sized), "fs_cluster_used" (CTAs per chain of the last
+ * small-width HMC launch: 1, 2, 4 or 8; 0 before the first) */
 int pyb_get_info(const pyb_handle* h, const char* key, double* value_out);
 
 /* ---- inputs ---- */
