@@ -67,6 +67,9 @@ SIGNATURES = {
     "pyb_hmc_adapt_end": [_P],
     "pyb_hmc_step_sizes": [_P, _f64p],
     "pyb_hmc_set_step_sizes": [_P, _f64p],
+    "pyb_hmc_set_temperatures": [_P, _f64p, C.c_int32],
+    "pyb_hmc_tempering_stats": [_P, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p],
+    "pyb_hmc_last_swaps": [_P, _f32p, _i32p],
     "pyb_hmc_track_predictive": [_P, _f32p, C.c_int64, _i32p],
     "pyb_hmc_predictive_sums": [_P, _f64p, _f64p, C.POINTER(C.c_int64)],
     "pyb_hmc_predictive_finish": [_P, _f64p, _f64p, C.c_int64, C.c_int64, C.c_int32, C.c_double, _f32p, _f32p, _f32p,

@@ -233,6 +233,8 @@ int pyb_set_option(pyb_handle* h, const char* key, double v) {
   } else if (!strcmp(key, "hmc_carry")) {
     h->opt_hmc_carry = v != 0;
     h->hmc.have_cur = false;
+  } else if (!strcmp(key, "hmc_swap")) {
+    h->opt_hmc_swap = v != 0;
   } else if (!strcmp(key, "hmc_keep_samples")) {
     PYB_REQUIRE(!h->hmc.sampling_started, PYB_ERR_STATE,
                 "hmc_keep_samples cannot change during a sampling phase (set it before, or after pyb_hmc_reset_samples)");
@@ -606,6 +608,31 @@ int pyb_hmc_set_step_sizes(pyb_handle* h, const double* eps) {
   PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
   use_device(h);
   hmc_set_step_sizes(h, eps);
+  PYB_CATCH
+}
+
+int pyb_hmc_set_temperatures(pyb_handle* h, const double* beta, int32_t R) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_set_temperatures(h, beta, R);
+  PYB_CATCH
+}
+
+int pyb_hmc_tempering_stats(pyb_handle* h, int64_t* rung_accepted, int64_t* rung_total, int64_t* swap_attempted,
+                            int64_t* swap_accepted) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_tempering_stats(h, rung_accepted, rung_total, swap_attempted, swap_accepted);
+  PYB_CATCH
+}
+
+int pyb_hmc_last_swaps(pyb_handle* h, float* log_r, int32_t* swapped) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_last_swaps(h, log_r, swapped);
   PYB_CATCH
 }
 

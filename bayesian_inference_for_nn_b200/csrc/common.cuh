@@ -100,7 +100,7 @@ struct Model {
 // ------------------------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al. 2011).  counter = (block, chain, iteration, stream), key = seed.
 // ------------------------------------------------------------------------------------------
-enum { STREAM_MOMENTUM = 0, STREAM_UNIFORM = 1, STREAM_INIT = 2, STREAM_SGLD = 3 };
+enum { STREAM_MOMENTUM = 0, STREAM_UNIFORM = 1, STREAM_INIT = 2, STREAM_SGLD = 3, STREAM_SWAP = 4 };
 
 __host__ __device__ inline void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,
                                                uint32_t k0, uint32_t k1, uint32_t out[4]) {
@@ -241,11 +241,23 @@ struct HmcState {
   bool adapting = false;
   int64_t adapt_t = 0;          // adaptation iterations run since pyb_hmc_adapt_begin
   double adapt_target = 0;
+  // parallel tempering (pyb_hmc_set_temperatures): local chain s = g R + r is rung r of replica group g; R = 0: off
+  int R = 0;
+  std::vector<double> ladder;   // [R] inverse temperatures, ladder[0] = 1
+  DevBuf<float> beta;           // [S] (float) inverse temperature of every chain's rung
+  DevBuf<double> ladder_d;      // [R] the ladder in double (swap ratios)
+  DevBuf<float> swap_logr;      // [S] log ratio of the swap proposed with the upper neighbour (NaN: none)
+  DevBuf<int32_t> swapped;      // [S] that swap was taken
+  DevBuf<int32_t> moved;        // [S] the position changed in this iteration: HMC accept or swap
+  DevBuf<unsigned long long> tcount;   // [4 R]: rung accepted, rung total, swaps attempted, swaps accepted
+  DevBuf<float> cold;           // [S / R, P] rung-0 positions gathered for the tracked predictive
+  bool swaps_ran = false;       // swap_logr / swapped hold an iteration's values
   // streamed posterior predictive (hmc_predictive.cu): the outputs o of every tracked draw on the tracked inputs
   struct Track {
     bool on = false;
     int64_t Nt = 0, chunk = 0;
     int64_t T = 0;              // draws per chain so far
+    int64_t nch = 0;            // tracked chains: S, or the S / R rung-0 chains of a tempering ladder
     DevBuf<float> x;            // [Nt, in_dim] library-owned copy of the inputs
     DevBuf<int32_t> y;          // [Nt] labels (empty: none given)
     DevBuf<float> out;          // [chunk, Nt, C] forward outputs of one chain chunk
@@ -365,6 +377,7 @@ struct pyb_handle {
   int opt_live_fused = 1;   // 1: the reference-live SVGD sweep is one cooperative launch on a single GPU
   int opt_hmc_carry = 1;    // 1: loss and gradient at the current position are carried to the next HMC iteration
   int opt_hmc_keep_samples = 1;   // 1: every tracked HMC draw is recorded (arena + host copy); 0: nothing is kept
+  int opt_hmc_swap = 1;     // 1: a tempering ladder proposes replica swaps every iteration; 0: the rungs run side by side
   int opt_predict_sharded = 0;   // 1: pyb_predict all-reduces its moment sums over the handle's communicator
   int opt_tc_fuse = 1;   // 1: layer 2 (+ loss, dZ2, dZ1) runs inside the layer-1 GEMM's epilogue where it applies
   int opt_tc_timeline = 0;   // diagnostics: the fused mma kernel records per-CTA cycle sums of its phases (info "tc_timeline_<k>")
@@ -480,6 +493,9 @@ void hmc_adapt_begin(pyb_handle* h, double target);
 void hmc_adapt_end(pyb_handle* h);
 void hmc_step_sizes(pyb_handle* h, double* out);
 void hmc_set_step_sizes(pyb_handle* h, const double* eps);
+void hmc_set_temperatures(pyb_handle* h, const double* beta, int R);
+void hmc_tempering_stats(pyb_handle* h, int64_t* rung_acc, int64_t* rung_tot, int64_t* swap_att, int64_t* swap_acc);
+void hmc_last_swaps(pyb_handle* h, float* log_r, int32_t* swapped);
 
 // svgd.cu
 void svgd_init(pyb_handle* h, int64_t S, int64_t offset, double lr, int sem, const double* p0);
@@ -537,7 +553,8 @@ bool is_device_ptr(const void* ptr);
 void hmc_track_start(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y);
 void hmc_track_stop(pyb_handle* h);
 void hmc_track_clear(pyb_handle* h);
-void hmc_track_draw(pyb_handle* h);
+void hmc_track_draw(pyb_handle* h, const float* q, int64_t n);
+void hmc_track_resize(pyb_handle* h);
 void hmc_track_sums(pyb_handle* h, double* sums, double* s2, int64_t* n_draws);
 void hmc_track_finish(pyb_handle* h, const double* sums, const double* s2, int64_t n_chains, int64_t n_draws,
                       const UncertaintyReq* uq, float* mean, float* var, float* rhat);

@@ -70,6 +70,7 @@ void fused_small_hmc_iteration(pyb_handle* h, bool burning) {
   p.eps = c.eps; p.half_eps = c.half; p.drift = c.drift;
   p.step = st.step.p; p.m = st.m;
   p.da = st.adapting ? st.da.p : nullptr; p.da_target = st.adapt_target; p.da_t = st.adapt_t;
+  p.beta = st.R ? st.beta.p : nullptr;
   p.stdv = (st.semantics == PYB_HMC_REFERENCE) ? (float)st.m : (float)sqrt(st.m);
   p.inv2m = (float)(1.0 / (2.0 * st.m));
   p.prior_const = (float)h->prior_const;

@@ -43,6 +43,7 @@ struct FsParams {
   float eps, half_eps, drift, stdv, inv2m, prior_const;
   double* step; double m;        // step != NULL: per-chain step sizes replace eps / half_eps / drift
   double* da; double da_target; int64_t da_t;   // da != NULL: adaptation iteration da_t (dual_average)
+  const float* beta;             // != NULL: tempering ladder, the chain's inverse temperature scales the data term
   int L, semantics, burning;
   int cluster;                   // CTAs per chain (1, 2, 4 or 8)
   uint64_t seed; uint32_t iter; int64_t chain_offset;
@@ -58,7 +59,7 @@ struct FsSmem {
   float* part;    // [n_slices][H*(D+1+C)]
   float* gx;      // [2][GX] cluster exchange: partial gradient [P] + loss sum (double) of this CTA's rows
   double* red;    // [32]
-  float* kc;      // [4] leapfrog coefficients of the chain's step size: full kick, half kick, drift
+  float* kc;      // [4] leapfrog coefficients of the chain's step size: full kick, half kick, drift; inverse temperature
 };
 
 template <typename T>
@@ -441,11 +442,13 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
   const int64_t s = blockIdx.x / n_ctas, P = p.P;
   const int t = threadIdx.x;
   const bool writer = rank == 0;          // every CTA of the cluster holds the same state; one writes it back
-  // the chain's leapfrog coefficients, kept in shared memory rather than in three registers for the whole kernel; the
-  // per-chain step size is read here, before the writer's Metropolis tail may update it (adaptation)
+  // the chain's leapfrog coefficients and inverse temperature (1 without a ladder; beta g rounds to g exactly), kept in
+  // shared memory rather than in registers for the whole kernel; the per-chain step size is read here, before the
+  // writer's Metropolis tail may update it (adaptation)
   if (t == 0) {
     const StepCoef c = p.step ? step_coef(p.step[s], p.m) : StepCoef{p.eps, p.half_eps, p.drift};
     sm.kc[0] = c.eps; sm.kc[1] = c.half; sm.kc[2] = c.drift;
+    sm.kc[3] = p.beta ? p.beta[s] : 1.f;
   }
   int n_eval = 0;
   auto eval = [&]() -> float {
@@ -470,12 +473,12 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
   // U0 and the first half kick share the evaluation at q0 (HMC.py:80-82)
   const float loss0 = eval();
   double e0 = 0.0;
-  const float half_eps0 = sm.kc[1], drift0 = sm.kc[2];
+  const float half_eps0 = sm.kc[1], drift0 = sm.kc[2], beta0 = sm.kc[3];
   for (int64_t i = t; i < P; i += FS_THREADS) {
     float q = sm.qs[i], d = q - p.mu[i], iv = p.inv_var[i];
     e0 += 0.5 * (double)(d * d * iv);
     if (writer) p.q0[s * P + i] = q;
-    float pp = sm.ps[i] - half_eps0 * (sm.gs[i] + d * iv);
+    float pp = sm.ps[i] - half_eps0 * (__fmul_rn(beta0, sm.gs[i]) + d * iv);
     sm.ps[i] = pp;
     sm.qs[i] = q + drift0 * pp;
   }
@@ -483,11 +486,11 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
   float loss1 = loss0, Up1 = 0.f, K1 = 0.f;
   for (int step = 1; step <= p.L; ++step) {
     loss1 = eval();
-    const float eps = sm.kc[0], half_eps = sm.kc[1], drift = sm.kc[2];
+    const float eps = sm.kc[0], half_eps = sm.kc[1], drift = sm.kc[2], beta = sm.kc[3];
     if (step < p.L) {
       for (int64_t i = t; i < P; i += FS_THREADS) {
         float q = sm.qs[i], d = q - p.mu[i];
-        float pp = sm.ps[i] - eps * (sm.gs[i] + d * p.inv_var[i]);
+        float pp = sm.ps[i] - eps * (__fmul_rn(beta, sm.gs[i]) + d * p.inv_var[i]);
         sm.ps[i] = pp;
         sm.qs[i] = q + drift * pp;
       }
@@ -496,7 +499,7 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
       double e1 = 0.0, k1 = 0.0;
       for (int64_t i = t; i < P; i += FS_THREADS) {
         float q = sm.qs[i], d = q - p.mu[i], iv = p.inv_var[i];
-        float gt = sm.gs[i] + d * iv;
+        float gt = __fmul_rn(beta, sm.gs[i]) + d * iv;
         e1 += 0.5 * (double)(d * d * iv);
         float pp = sm.ps[i];
         if (p.semantics == PYB_HMC_REFERENCE) {   // L-th full kick, then the trailing half kick (HMC.py:85-87)
@@ -520,8 +523,9 @@ __global__ void __launch_bounds__(FS_THREADS, 4) k_fs_hmc(FsParams p) {
   if (n_ctas > 1) cooperative_groups::this_cluster().sync();     // nobody leaves while a peer may still read its shared memory
   if (t == 0 && writer) {
     // Metropolis test (HMC.py:91), same expression order as k_accept
-    float U0 = (Up0 + p.prior_const) + loss0 * p.n_train;
-    float U1 = (Up1 + p.prior_const) + loss1 * p.n_train;
+    const float tl0 = __fmul_rn(sm.kc[3], loss0), tl1 = __fmul_rn(sm.kc[3], loss1);
+    float U0 = (Up0 + p.prior_const) + tl0 * p.n_train;
+    float U1 = (Up1 + p.prior_const) + tl1 * p.n_train;
     float la = ((K0 + U0) - K1) - U1;
     float alpha = expf(la);
     float u = p.inj_u ? p.inj_u[s] : philox_uniform((uint32_t)(p.chain_offset + s), p.iter, STREAM_UNIFORM, p.seed);

@@ -104,7 +104,7 @@ void hmc_track_stop(pyb_handle* h) {
   for (DevBuf<double>* b : {&t.s1c, &t.Q, &t.Qd, &t.S2, &t.part}) b->release();
   t.y.release();
   t.on = false;
-  t.Nt = t.chunk = t.T = 0;
+  t.Nt = t.chunk = t.T = t.nch = 0;
 }
 
 void hmc_track_clear(pyb_handle* h) {
@@ -124,7 +124,7 @@ void hmc_track_start(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y
               "the predictive must be tracked from the first sampling iteration on: call before it (or after pyb_hmc_reset_samples)");
   PYB_REQUIRE(Nt > 0, PYB_ERR_INVALID, "Nt must be > 0");
   const Model& m = h->model;
-  const int64_t C = m.out_dim, elems = Nt * C, S = st.S;
+  const int64_t C = m.out_dim, elems = Nt * C, S = st.R ? st.S / st.R : st.S;   // a ladder tracks its rung-0 chains only
   const int Ce = C == 1 ? 2 : (int)C;
   if (y) {
     PYB_REQUIRE(Ce * Ce <= 1024, PYB_ERR_UNSUPPORTED, "classification uncertainty supports at most 32 classes");
@@ -168,6 +168,7 @@ void hmc_track_start(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y
   if (s2) t.S2.alloc((size_t)Nt * C * C);
   t.part.alloc((size_t)ngroups * 2 * elems);
   t.Nt = Nt;
+  t.nch = S;
   t.chunk = chunk;
   t.on = true;
   tc_invalidate_track(h);
@@ -175,18 +176,39 @@ void hmc_track_start(pyb_handle* h, const float* x, int64_t Nt, const int32_t* y
   PYB_CUDA(cudaStreamSynchronize(h->stream));
 }
 
-// one draw per chain: the chains' current positions st.q (enqueued on the handle's stream, no host sync)
-void hmc_track_draw(pyb_handle* h) {
+// a tempering ladder set or cleared after tracking started (no draw tracked yet): the per-chain sums follow the number
+// of tracked chains
+void hmc_track_resize(pyb_handle* h) {
+  HmcState& st = h->hmc;
+  HmcState::Track& t = st.track;
+  if (!t.on) return;
+  const int64_t n = st.R ? st.S / st.R : st.S, elems = t.Nt * h->model.out_dim;
+  if (n > t.chunk) {             // the chunk was sized for fewer chains: size it again as hmc_track_start would
+    int64_t chunk = generic_chain_batch(h, n, t.Nt, false);
+    chunk = std::min<int64_t>(chunk, std::max<int64_t>(1, (int64_t)((512ull << 20) / (sizeof(float) * (size_t)elems))));
+    t.chunk = std::max(t.chunk, chunk);
+    t.out.alloc((size_t)t.chunk * elems);
+    t.part.alloc((size_t)((t.chunk + kTrackGroup - 1) / kTrackGroup) * 2 * elems);
+  }
+  t.shift.alloc((size_t)n * elems);
+  t.s1c.alloc((size_t)n * elems);
+  t.nch = n;
+  hmc_track_clear(h);
+}
+
+// one draw per chain of the n positions q [n, P] (st.q, or the gathered rung-0 chains of a ladder), enqueued on the
+// handle's stream, no host sync
+void hmc_track_draw(pyb_handle* h, const float* q, int64_t n) {
   NvtxRange nv("pyb.hmc.track_predictive");
   HmcState& st = h->hmc;
   HmcState::Track& t = st.track;
   const Model& m = h->model;
-  const int64_t P = m.P, C = m.out_dim, Nt = t.Nt, elems = Nt * C, S = st.S;
+  const int64_t P = m.P, C = m.out_dim, Nt = t.Nt, elems = Nt * C, S = n;
   const bool tensor = track_tensor(h, Nt);
   for (int64_t b0 = 0; b0 < S; b0 += t.chunk) {
     const int64_t nb = std::min(t.chunk, S - b0);
-    if (tensor) tc_forward_tracked(h, st.q.p + b0 * P, nb, t.x.p, Nt, t.out.p);
-    else generic_forward(h, st.q.p + b0 * P, nb, t.x.p, Nt, t.out.p);
+    if (tensor) tc_forward_tracked(h, q + b0 * P, nb, t.x.p, Nt, t.out.p);
+    else generic_forward(h, q + b0 * P, nb, t.x.p, Nt, t.out.p);
     const int ngroups = (int)((nb + kTrackGroup - 1) / kTrackGroup);
     dim3 g((unsigned)((elems + 255) / 256), (unsigned)ngroups);
     k_track_accum<<<g, 256, 0, h->stream>>>(t.out.p, nb, elems, t.T == 0 ? 1 : 0, t.shift.p + b0 * elems,
@@ -207,7 +229,7 @@ void hmc_track_sums(pyb_handle* h, double* sums, double* s2, int64_t* n_draws) {
   const int64_t elems = t.Nt * h->model.out_dim;
   DevBuf<double> amw;
   amw.alloc(3 * (size_t)elems);
-  k_track_reduce<<<(unsigned)((elems + 255) / 256), 256, 0, h->stream>>>(t.shift.p, t.s1c.p, t.Qd.p, st.S, elems,
+  k_track_reduce<<<(unsigned)((elems + 255) / 256), 256, 0, h->stream>>>(t.shift.p, t.s1c.p, t.Qd.p, t.nch, elems,
                                                                          (double)t.T, amw.p, amw.p + elems, amw.p + 2 * elems);
   count_launch(h);
   const size_t eb = elems * sizeof(double);

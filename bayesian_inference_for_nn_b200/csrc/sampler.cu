@@ -79,7 +79,8 @@ __global__ void k_finish(const double* partial, int nblk, double scale, float* o
 //   [kinetic]  partial_k += p^2                    (HMC.py:161-166)
 //   q += drift*p   (drift==0: skipped)             (HMC.py:138-141)
 // The coefficients are the scalars kick1 / kick2 / drift, or, with per-chain step sizes (step != NULL), those of the
-// block's chain for the leapfrog position `role`.
+// block's chain for the leapfrog position `role`.  With a tempering ladder (beta != NULL) the data gradient g is scaled
+// by the chain's inverse temperature first: gtot = beta g + (q-mu)/sigma^2 (beta = 1 rounds exactly as without).
 enum KickRole {
   KICK_HALF_DRIFT,   // first half kick + drift (HMC.py:82-83)
   KICK_FULL_DRIFT,   // full kick + drift (:84-85)
@@ -97,6 +98,7 @@ struct KickArgs {
   int64_t P, S;
   float kick1, kick2, drift;
   const double* step; double m; int role;
+  const float* beta;
   int snapshot, energy, kinetic;
   double* partial_e; double* partial_k;
 };
@@ -105,6 +107,7 @@ __global__ void __launch_bounds__(EW_THREADS) k_kick_drift(KickArgs a) {
   int64_t s = chain_index();
   if (s >= a.S) return;
   if (a.step) kick_coefs(a.role, step_coef(a.step[s], a.m), a.kick1, a.kick2, a.drift);
+  const float b = a.beta ? a.beta[s] : 1.f;
   int64_t base = (int64_t)blockIdx.x * EW_CHUNK + threadIdx.x;
   double e = 0.0, k = 0.0;
 #pragma unroll
@@ -115,7 +118,7 @@ __global__ void __launch_bounds__(EW_THREADS) k_kick_drift(KickArgs a) {
       float q = a.q[o], p = a.p[o];
       float d = q - a.mu[i];
       float iv = a.inv_var[i];
-      float gt = a.g[o] + d * iv;
+      float gt = __fmul_rn(b, a.g[o]) + d * iv;
       if (a.energy) e += 0.5 * (double)(d * d * iv);
       if (a.snapshot) a.q0[o] = q;
       p = p - a.kick1 * gt;
@@ -163,7 +166,8 @@ __global__ void k_potential(const float* Up, const float* loss, float prior_cons
   if (s < S) U[s] = (Up[s] + prior_const) + loss[s] * n_train;
 }
 
-// Metropolis test (HMC.py:91): accept iff burning or u < exp(K0+U0-K1-U1); NaN => reject.
+// Metropolis test (HMC.py:91): accept iff burning or u < exp(K0+U0-K1-U1); NaN => reject.  With a tempering ladder
+// (beta != NULL) the data term of U is the chain's beta times the mean loss times n_train; ret_loss stays untempered.
 struct AcceptArgs {
   const float* Up0; const float* Up1; const float* loss0; const float* loss1; const float* K0; const float* K1;
   float prior_const, n_train;
@@ -173,6 +177,7 @@ struct AcceptArgs {
   float* U0; float* U1; float* log_alpha; int32_t* accepted; float* ret_loss;
   unsigned long long* counters; double* loss_sum;
   double* da; double* step; double da_target; int64_t da_t;   // da != NULL: adaptation iteration da_t (dual_average)
+  const float* beta;
 };
 __global__ void k_accept(AcceptArgs a) {
   __shared__ double scratch[32];
@@ -180,8 +185,10 @@ __global__ void k_accept(AcceptArgs a) {
   double ls = 0.0;
   int acc = 0, isnan_ = 0;
   if (s < a.S) {
-    float U0 = (a.Up0[s] + a.prior_const) + a.loss0[s] * a.n_train;
-    float U1 = (a.Up1[s] + a.prior_const) + a.loss1[s] * a.n_train;
+    float l0 = a.loss0[s], l1 = a.loss1[s];
+    if (a.beta) { l0 = __fmul_rn(a.beta[s], l0); l1 = __fmul_rn(a.beta[s], l1); }
+    float U0 = (a.Up0[s] + a.prior_const) + l0 * a.n_train;
+    float U1 = (a.Up1[s] + a.prior_const) + l1 * a.n_train;
     float la = ((a.K0[s] + U0) - a.K1[s]) - U1;
     float alpha = expf(la);
     float u = a.inj_u ? a.inj_u[s] : philox_uniform((uint32_t)(a.chain_offset + s), a.iter, STREAM_UNIFORM, a.seed);
@@ -207,18 +214,19 @@ __global__ void k_accept(AcceptArgs a) {
 
 // Sample bookkeeping (HMC.py:75-77, 92-96, 103): single block; slot order = chain order, so the
 // arena layout is deterministic.  first!=0: every chain first records its pre-iteration state
-// with frequency 1.
+// with frequency 1.  The recording chains are s = k stride, k < S (stride R: the rung-0 chains of a tempering ladder,
+// with accepted = "moved": HMC accept or swap).
 __global__ void __launch_bounds__(1024) k_record_slots(const int32_t* accepted, int64_t S, int first,
                                                         int32_t* arena_count, int32_t* arena_freq,
                                                         int32_t* arena_chain, int32_t* last_idx,
                                                         int32_t* pending_freq, int32_t* slot_first,
-                                                        int32_t* slot_acc, int64_t chain_offset) {
+                                                        int32_t* slot_acc, int64_t chain_offset, int64_t stride) {
   __shared__ int tot[1024];
   const int t = threadIdx.x;
   const int64_t cpt = (S + blockDim.x - 1) / blockDim.x;
   const int64_t lo = (int64_t)t * cpt, hi = (lo + cpt < S) ? lo + cpt : S;
   int need = 0;
-  for (int64_t s = lo; s < hi; ++s) need += (first ? 1 : 0) + (accepted[s] ? 1 : 0);
+  for (int64_t k = lo; k < hi; ++k) need += (first ? 1 : 0) + (accepted[k * stride] ? 1 : 0);
   tot[t] = need;
   __syncthreads();
   // Hillis-Steele inclusive scan over the 1024 per-thread totals
@@ -229,7 +237,8 @@ __global__ void __launch_bounds__(1024) k_record_slots(const int32_t* accepted, 
     __syncthreads();
   }
   int slot = *arena_count + tot[t] - need;
-  for (int64_t s = lo; s < hi; ++s) {
+  for (int64_t k = lo; k < hi; ++k) {
+    const int64_t s = k * stride;
     int sf = -1, sa = -1;
     if (first) {
       sf = slot++;
@@ -276,6 +285,99 @@ __global__ void __launch_bounds__(EW_THREADS) k_select_record(float* q, const fl
       if (!acc) q[o] = old;
       if (sa >= 0) arena[(int64_t)sa * P + i] = cur;
       if (gcur && acc) gcur[o] = g[o];
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------
+// replica exchange (parallel tempering): one deterministic even-odd swap round per iteration (Syed, Bouchard-Cote,
+// Deligiannidis & Doucet 2022).  Chain s = g R + r is rung r of group g; in iteration `iter` the pairs (r, r + 1) with
+// r = iter (mod 2) of every group propose to exchange their states, accepted iff u < exp(log_r) with
+//   log_r = (beta_r - beta_{r+1}) n_train (loss_r - loss_{r+1})   (double; NaN rejects)
+// and u the Philox uniform of the lower chain's global id on STREAM_SWAP.
+// ------------------------------------------------------------------------------------------
+constexpr int kMaxRungs = 64;
+
+// One thread per chain.  The lower chain of a proposed pair decides for the pair, exchanges the two untempered losses
+// ret_loss (with carry on they become the carried losses) and writes both chains' "moved" flags; every chain reports
+// the swap it proposed with its upper neighbour (log_r / swapped: NaN / 0 when none).  propose = 0 (option hmc_swap)
+// keeps the rungs apart and only counts.  tcount [4 R] += per rung: HMC accepts, chains, swaps attempted / accepted
+// (lower rung of the pair).
+__global__ void __launch_bounds__(256) k_swap_decide(const double* ladder, int R, int propose, double n_train,
+                                                      uint64_t seed, uint32_t iter, int64_t chain_offset, int64_t S,
+                                                      const int32_t* accepted, float* ret_loss, float* log_r,
+                                                      int32_t* swapped, int32_t* moved, unsigned long long* tcount) {
+  __shared__ unsigned cnt[4 * kMaxRungs];
+  for (int i = threadIdx.x; i < 4 * R; i += blockDim.x) cnt[i] = 0u;
+  __syncthreads();
+  const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s < S) {
+    const int r = (int)(s % R), par = (int)(iter & 1u);
+    const bool lower = propose && r + 1 < R && (r & 1) == par;
+    const bool upper = propose && r >= 1 && ((r - 1) & 1) == par;
+    const int acc = accepted[s];
+    float lr_out = NAN;
+    int sw = 0;
+    if (lower) {
+      const float l0 = ret_loss[s], l1 = ret_loss[s + 1];
+      const double lr = (ladder[r] - ladder[r + 1]) * n_train * ((double)l0 - (double)l1);
+      const float u = philox_uniform((uint32_t)(chain_offset + s), iter, STREAM_SWAP, seed);
+      sw = ((double)u < exp(lr)) ? 1 : 0;
+      lr_out = (float)lr;
+      if (sw) { ret_loss[s] = l1; ret_loss[s + 1] = l0; }
+      moved[s] = acc | sw;
+      moved[s + 1] = accepted[s + 1] | sw;
+      atomicAdd(&cnt[2 * R + r], 1u);
+      if (sw) atomicAdd(&cnt[3 * R + r], 1u);
+    } else if (!upper) {
+      moved[s] = acc;
+    }
+    log_r[s] = lr_out;
+    swapped[s] = sw;
+    if (acc) atomicAdd(&cnt[r], 1u);
+    atomicAdd(&cnt[R + r], 1u);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < 4 * R; i += blockDim.x)
+    if (cnt[i]) atomicAdd(&tcount[i], (unsigned long long)cnt[i]);
+}
+
+// the accepted swaps: chains s (swapped[s]) and s + 1 exchange their positions and, with carry on, the loss gradients
+// carried with them; momenta are redrawn every iteration and step sizes stay with the chain slot
+__global__ void __launch_bounds__(EW_THREADS) k_swap_exchange(float* q, float* gcur, const int32_t* swapped, int64_t P,
+                                                               int64_t S) {
+  const int64_t s = chain_index();
+  if (s >= S || !swapped[s]) return;
+  const int64_t base = (int64_t)blockIdx.x * EW_CHUNK + threadIdx.x;
+#pragma unroll
+  for (int j = 0; j < EW_PER_THREAD; ++j) {
+    const int64_t i = base + (int64_t)j * EW_THREADS;
+    if (i < P) {
+      const int64_t a = s * P + i, b = a + P;
+      const float qa = q[a], qb = q[b];
+      q[a] = qb; q[b] = qa;
+      if (gcur) { const float ga = gcur[a], gb = gcur[b]; gcur[a] = gb; gcur[b] = ga; }
+    }
+  }
+}
+
+// arena rows of the rung-0 chains s = k R (k < G): the pre-iteration state q0 in the first sampling iteration, the
+// position after the swap when the chain moved
+__global__ void __launch_bounds__(EW_THREADS) k_record_cold(const float* q, const float* q0, const int32_t* slot_first,
+                                                             const int32_t* slot_acc, float* arena, int64_t P, int64_t R,
+                                                             int64_t G) {
+  const int64_t k = chain_index();
+  if (k >= G) return;
+  const int64_t s = k * R;
+  const int sf = slot_first[s], sa = slot_acc[s];
+  if (sf < 0 && sa < 0) return;
+  const int64_t base = (int64_t)blockIdx.x * EW_CHUNK + threadIdx.x;
+#pragma unroll
+  for (int j = 0; j < EW_PER_THREAD; ++j) {
+    const int64_t i = base + (int64_t)j * EW_THREADS;
+    if (i < P) {
+      if (sf >= 0) arena[(int64_t)sf * P + i] = q0[s * P + i];
+      if (sa >= 0) arena[(int64_t)sa * P + i] = q[s * P + i];
     }
   }
 }
@@ -328,6 +430,10 @@ void hmc_init(pyb_handle* h, int64_t S, int64_t chain_offset, double eps, double
   st.adapting = false;
   st.adapt_t = 0;
   st.step.release(); st.da.release();
+  st.R = 0; st.ladder.clear();        // pyb_hmc_init clears the tempering ladder
+  st.beta.release(); st.ladder_d.release(); st.swap_logr.release(); st.swapped.release(); st.moved.release();
+  st.tcount.release(); st.cold.release();
+  st.swaps_ran = false;
   hmc_track_stop(h);
   DevBuf<float> tmp;
   const float* q0d = nullptr;
@@ -399,6 +505,7 @@ static void launch_kick(pyb_handle* h, const float* g, KickRole role, bool snaps
   a.q = st.q.p; a.p = st.p.p; a.g = g; a.q0 = st.q0.p; a.mu = h->mu.p; a.inv_var = h->inv_var.p; a.P = P; a.S = st.S;
   kick_coefs(role, step_coef(st.eps, st.m), a.kick1, a.kick2, a.drift);
   a.step = st.step.p; a.m = st.m; a.role = role;
+  a.beta = st.R ? st.beta.p : nullptr;
   a.snapshot = snapshot; a.energy = energy; a.kinetic = kinetic;
   a.partial_e = st.partial_e.p; a.partial_k = st.partial_k.p;
   k_kick_drift<<<chain_grid(nblk, st.S), EW_THREADS, 0, h->stream>>>(a);
@@ -424,6 +531,49 @@ static bool update_i8_guard(pyb_handle* h, const float* loss_dev, int64_t S) {
   return ok;
 }
 
+// one tracked draw of every chain at its current position; a ladder tracks its rung-0 chains, gathered into [G, P]
+static void track_current(pyb_handle* h) {
+  HmcState& st = h->hmc;
+  const int64_t P = h->model.P;
+  if (!st.R) { hmc_track_draw(h, st.q.p, st.S); return; }
+  const int64_t G = st.S / st.R;
+  PYB_CUDA(cudaMemcpy2DAsync(st.cold.p, P * sizeof(float), st.q.p, st.R * P * sizeof(float), P * sizeof(float), G,
+                             cudaMemcpyDeviceToDevice, h->stream));
+  hmc_track_draw(h, st.cold.p, G);
+}
+
+// the end of a tempered iteration: restore the rejected chains (carrying the gradient of the accepted ones), one swap
+// round, then the rung-0 chains record a draw wherever they moved (HMC accept or swap)
+static void tempered_tail(pyb_handle* h, bool record, bool first, bool carry) {
+  HmcState& st = h->hmc;
+  const int64_t P = h->model.P, S = st.S, R = st.R, G = S / R;
+  const int nblk = ew_blocks(P);
+  k_select_record<<<chain_grid(nblk, S), EW_THREADS, 0, h->stream>>>(st.q.p, st.q0.p, st.accepted.p, st.slot_first.p,
+                                                                     st.slot_acc.p, st.arena.p, P, 0, S,
+                                                                     carry ? st.gcur.p : nullptr, st.g.p);
+  const int propose = h->opt_hmc_swap ? 1 : 0;
+  NvtxRange nv("pyb.hmc.swap");
+  k_swap_decide<<<(unsigned)((S + 255) / 256), 256, 0, h->stream>>>(st.ladder_d.p, (int)R, propose, (double)h->n_train,
+                                                                    h->seed, (uint32_t)st.iter, st.chain_offset, S,
+                                                                    st.accepted.p, st.ret_loss.p, st.swap_logr.p,
+                                                                    st.swapped.p, st.moved.p, st.tcount.p);
+  count_launch(h, 2);
+  if (propose) {
+    k_swap_exchange<<<chain_grid(nblk, S), EW_THREADS, 0, h->stream>>>(st.q.p, carry ? st.gcur.p : nullptr,
+                                                                       st.swapped.p, P, S);
+    count_launch(h);
+  }
+  st.swaps_ran = true;
+  if (record) {
+    k_record_slots<<<1, 1024, 0, h->stream>>>(st.moved.p, G, first ? 1 : 0, st.arena_count.p, st.arena_freq.p,
+                                              st.arena_chain.p, st.last_idx.p, st.pending_freq.p, st.slot_first.p,
+                                              st.slot_acc.p, st.chain_offset, R);
+    k_record_cold<<<chain_grid(nblk, G), EW_THREADS, 0, h->stream>>>(st.q.p, st.q0.p, st.slot_first.p, st.slot_acc.p,
+                                                                     st.arena.p, P, R, G);
+    count_launch(h, 2);
+  }
+}
+
 void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_diag* out) {
   HmcState& st = h->hmc;
   PYB_REQUIRE(st.inited, PYB_ERR_STATE, "pyb_hmc_init must be called first");
@@ -437,6 +587,7 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
   int64_t launches0 = h->kernel_launches;
   PYB_CUDA(cudaMemsetAsync(st.counters.p, 0, 4 * sizeof(unsigned long long), h->stream));
   PYB_CUDA(cudaMemsetAsync(st.loss_sum.p, 0, sizeof(double), h->stream));
+  if (st.R) PYB_CUDA(cudaMemsetAsync(st.tcount.p, 0, st.tcount.bytes(), h->stream));
   PYB_CUDA(cudaEventRecord(h->ev0, h->stream));
   const int path = resolve_path(h, S, true);
   int64_t evals = 0;
@@ -447,12 +598,12 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
     bool first = sampling && !st.sampling_started;
     const bool record = sampling && h->opt_hmc_keep_samples;   // keep the draws (arena), not only the tracked sums
     if (record) {
-      int64_t need = S * (first ? 2 : 1);
+      int64_t need = (st.R ? S / st.R : S) * (first ? 2 : 1);    // a ladder records its rung-0 chains only
       if (!st.arena.p) hmc_size_arena(h);
       if (st.arena_used_upper + need > st.arena_cap) hmc_flush_arena(h);
       st.arena_used_upper += need;
     }
-    if (first && st.track.on) hmc_track_draw(h);     // the pre-iteration state is the first draw (HMC.py:75-77)
+    if (first && st.track.on) track_current(h);     // the pre-iteration state is the first draw (HMC.py:75-77)
     if (st.adapting) st.adapt_t++;
     dim3 gridp = chain_grid(nblk, S);
     if (path == PYB_PATH_FUSED_SMALL) {
@@ -501,22 +652,27 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
     a.U0 = st.U0.p; a.U1 = st.U1.p; a.log_alpha = st.log_alpha.p; a.accepted = st.accepted.p;
     a.ret_loss = st.ret_loss.p; a.counters = st.counters.p; a.loss_sum = st.loss_sum.p;
     a.da = st.adapting ? st.da.p : nullptr; a.step = st.step.p; a.da_target = st.adapt_target; a.da_t = st.adapt_t;
+    a.beta = st.R ? st.beta.p : nullptr;
     k_accept<<<(unsigned)((S + 255) / 256), 256, 0, h->stream>>>(a);
     count_launch(h);
     }
+    const bool carry = h->opt_hmc_carry && path != PYB_PATH_FUSED_SMALL;
+    if (st.R) {
+      tempered_tail(h, record, first, carry);
+    } else {
     if (record) {
       k_record_slots<<<1, 1024, 0, h->stream>>>(st.accepted.p, S, first ? 1 : 0, st.arena_count.p, st.arena_freq.p,
                                                 st.arena_chain.p, st.last_idx.p, st.pending_freq.p,
-                                                st.slot_first.p, st.slot_acc.p, st.chain_offset);
+                                                st.slot_first.p, st.slot_acc.p, st.chain_offset, 1);
       count_launch(h);
     }
-    if (sampling) st.sampling_started = true;
-    const bool carry = h->opt_hmc_carry && path != PYB_PATH_FUSED_SMALL;
     k_select_record<<<gridp, EW_THREADS, 0, h->stream>>>(st.q.p, st.q0.p, st.accepted.p, st.slot_first.p,
                                                          st.slot_acc.p, st.arena.p, P, record ? 1 : 0, S,
                                                          carry ? st.gcur.p : nullptr, st.g.p);
     count_launch(h);
-    if (sampling && st.track.on) hmc_track_draw(h);  // the post-accept position (HMC.py:92-104)
+    }
+    if (sampling) st.sampling_started = true;
+    if (sampling && st.track.on) track_current(h);  // the post-accept (post-swap) position (HMC.py:92-104)
     if (carry)     // loss at the new current position = what step() returns: accepted ? loss(q_L) : loss(q0) (HMC.py:96,104)
       PYB_CUDA(cudaMemcpyAsync(st.loss0.p, st.ret_loss.p, S * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
     st.have_cur = carry;
@@ -662,6 +818,74 @@ void hmc_set_step_sizes(pyb_handle* h, const double* eps) {
   st.step.alloc(st.S);
   PYB_CUDA(cudaMemcpyAsync(st.step.p, eps, st.S * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   PYB_CUDA(cudaStreamSynchronize(h->stream));
+}
+
+// ------------------------------------------------------------------------------------------
+// tempering ladder (parallel tempering / replica exchange)
+// ------------------------------------------------------------------------------------------
+void hmc_set_temperatures(pyb_handle* h, const double* beta, int R) {
+  HmcState& st = h->hmc;
+  require_inited(st);
+  PYB_REQUIRE(!st.sampling_started, PYB_ERR_STATE,
+              "the ladder cannot change during a sampling phase (set it after pyb_hmc_init or pyb_hmc_reset_samples)");
+  if (R == 0 && !beta) {
+    PYB_CUDA(cudaStreamSynchronize(h->stream));
+    st.R = 0; st.ladder.clear();
+    st.beta.release(); st.ladder_d.release(); st.swap_logr.release(); st.swapped.release(); st.moved.release();
+    st.tcount.release(); st.cold.release();
+    st.swaps_ran = false;
+    hmc_track_resize(h);
+    return;
+  }
+  PYB_REQUIRE(beta, PYB_ERR_INVALID, "beta is NULL (pass NULL with R = 0 to turn tempering off)");
+  PYB_REQUIRE(R >= 2 && R <= kMaxRungs, PYB_ERR_INVALID, "a ladder has 2 to 64 rungs");
+  PYB_REQUIRE(beta[0] == 1.0, PYB_ERR_INVALID, "the first inverse temperature must be 1");
+  for (int r = 1; r < R; ++r)
+    PYB_REQUIRE(isfinite(beta[r]) && beta[r] > 0.0 && beta[r] < beta[r - 1], PYB_ERR_INVALID,
+                "inverse temperatures must decrease strictly and stay > 0");
+  PYB_REQUIRE(st.S % R == 0, PYB_ERR_INVALID, "the number of local chains must be a multiple of the ladder length");
+  PYB_REQUIRE(st.chain_offset % R == 0, PYB_ERR_INVALID, "chain_offset must be a multiple of the ladder length");
+  const int64_t S = st.S, P = h->model.P;
+  std::vector<float> bs((size_t)S);
+  for (int64_t s = 0; s < S; ++s) bs[s] = (float)beta[s % R];
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
+  st.beta.alloc(S); st.ladder_d.alloc(R); st.swap_logr.alloc(S); st.swapped.alloc(S); st.moved.alloc(S);
+  st.tcount.alloc(4 * (size_t)R); st.cold.alloc((size_t)(S / R) * P);
+  PYB_CUDA(cudaMemcpy(st.beta.p, bs.data(), S * sizeof(float), cudaMemcpyHostToDevice));
+  PYB_CUDA(cudaMemcpy(st.ladder_d.p, beta, R * sizeof(double), cudaMemcpyHostToDevice));
+  PYB_CUDA(cudaMemset(st.tcount.p, 0, st.tcount.bytes()));
+  st.ladder.assign(beta, beta + R);
+  st.R = R;
+  st.swaps_ran = false;
+  hmc_track_resize(h);
+}
+
+void hmc_tempering_stats(pyb_handle* h, int64_t* rung_acc, int64_t* rung_tot, int64_t* swap_att, int64_t* swap_acc) {
+  HmcState& st = h->hmc;
+  require_inited(st);
+  PYB_REQUIRE(st.R, PYB_ERR_STATE, "no tempering ladder is set: call pyb_hmc_set_temperatures first");
+  const int R = st.R;
+  std::vector<unsigned long long> c(4 * (size_t)R);
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
+  PYB_CUDA(cudaMemcpy(c.data(), st.tcount.p, c.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  for (int r = 0; r < R; ++r) {
+    if (rung_acc) rung_acc[r] = (int64_t)c[r];
+    if (rung_tot) rung_tot[r] = (int64_t)c[R + r];
+    if (r + 1 < R) {
+      if (swap_att) swap_att[r] = (int64_t)c[2 * R + r];
+      if (swap_acc) swap_acc[r] = (int64_t)c[3 * R + r];
+    }
+  }
+}
+
+void hmc_last_swaps(pyb_handle* h, float* log_r, int32_t* swapped) {
+  HmcState& st = h->hmc;
+  require_inited(st);
+  PYB_REQUIRE(st.R, PYB_ERR_STATE, "no tempering ladder is set: call pyb_hmc_set_temperatures first");
+  PYB_REQUIRE(st.swaps_ran, PYB_ERR_STATE, "no iteration has run under this ladder yet");
+  PYB_CUDA(cudaStreamSynchronize(h->stream));
+  if (log_r) PYB_CUDA(cudaMemcpy(log_r, st.swap_logr.p, st.S * sizeof(float), cudaMemcpyDeviceToHost));
+  if (swapped) PYB_CUDA(cudaMemcpy(swapped, st.swapped.p, st.S * sizeof(int32_t), cudaMemcpyDeviceToHost));
 }
 
 }  // namespace pyb

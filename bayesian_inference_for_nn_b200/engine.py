@@ -115,6 +115,7 @@ class Engine:
         check(self.lib.pyb_hmc_init(self.h, int(S), int(chain_offset), float(eps), float(m), int(L), int(semantics),
                                     _ptr(q0a)))
         self.S = int(S)
+        self.R = 1                      # pyb_hmc_init clears any tempering ladder
         self._track = None
 
     def hmc_inject(self, p=None, u=None):
@@ -186,6 +187,37 @@ class Engine:
         if e.shape[0] != self.S:
             raise ValueError("expected %d step sizes, got %d" % (self.S, e.shape[0]))
         check(self.lib.pyb_hmc_set_step_sizes(self.h, _ptr(e)))
+
+    # ---- parallel tempering (pyb_hmc_set_temperatures, pyb_hmc_tempering_stats, pyb_hmc_last_swaps)
+    def hmc_set_temperatures(self, beta):
+        """Run the S chains as S / R replica groups over the ladder ``beta`` (R inverse temperatures, beta[0] = 1,
+        strictly decreasing, > 0): chain g R + r is rung r of group g; only rung 0 records draws.  None turns tempering
+        off.  Call after ``hmc_init`` and before the first sampling iteration."""
+        if beta is None:
+            check(self.lib.pyb_hmc_set_temperatures(self.h, None, 0))
+            self.R = 1
+            return
+        b = np.ascontiguousarray(beta, dtype=np.float64).reshape(-1)
+        check(self.lib.pyb_hmc_set_temperatures(self.h, _ptr(b), int(b.shape[0])))
+        self.R = int(b.shape[0])
+
+    def hmc_tempering_stats(self):
+        """counts of the last ``hmc_run`` over this engine's groups: per rung HMC proposals accepted / made
+        ([R] int64), per pair (r, r + 1) swaps attempted / accepted ([R - 1] int64)"""
+        R = self.R
+        out = dict(rung_accepted=np.zeros(R, np.int64), rung_total=np.zeros(R, np.int64),
+                   swap_attempted=np.zeros(R - 1, np.int64), swap_accepted=np.zeros(R - 1, np.int64))
+        check(self.lib.pyb_hmc_tempering_stats(self.h, _ptr(out["rung_accepted"]), _ptr(out["rung_total"]),
+                                               _ptr(out["swap_attempted"]), _ptr(out["swap_accepted"])))
+        return out
+
+    def hmc_last_swaps(self):
+        """-> (log_r [S] float32, swapped [S] bool): the swap each chain proposed with its upper neighbour in the
+        last iteration (NaN / False where none)"""
+        lr = np.empty(self.S, np.float32)
+        sw = np.empty(self.S, np.int32)
+        check(self.lib.pyb_hmc_last_swaps(self.h, _ptr(lr), _ptr(sw)))
+        return lr, sw.astype(bool)
 
     # ---- streamed HMC predictive (pyb_hmc_track_predictive / _sums / _finish)
     def hmc_track_predictive(self, x, y=None):

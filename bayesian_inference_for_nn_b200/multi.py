@@ -6,7 +6,9 @@ process, each driven by its own host thread (every C call releases the GIL, so t
 
 * HMC chains never interact: device i owns the global chains [lo_i, hi_i) (``sharding.shard_range``) and is initialised
   with ``chain_offset=lo_i``, so the Philox counters — and therefore every trajectory and every sample — are those of the
-  one-device run; ``result()`` pools the per-device samples in global chain order.
+  one-device run; ``result()`` pools the per-device samples in global chain order.  With a tempering ladder of R rungs
+  the unit of sharding is the replica group: device i owns groups [lo_i, hi_i), i.e. chains [R lo_i, R hi_i), and swaps
+  stay inside a device.
 * SVGD particles: each engine joins one NCCL communicator (``pyb_svgd_set_comm``) and the exchange step runs inside the
   library (svgd.cu); the engines must hold the same number of particles.
 """
@@ -61,7 +63,12 @@ class EngineGroup:
             self._pool = None
 
     # ---- HMC ------------------------------------------------------------------------------------------------------
-    def hmc_init(self, n_chains, eps, m, L, semantics, q0=None, chain_offset=0):
+    def hmc_init(self, n_chains, eps, m, L, semantics, q0=None, chain_offset=0, ladder=None):
+        """n_chains posterior chains; with ``ladder`` (R inverse temperatures) each is a replica group of R engine
+        chains, q0 rows (one per posterior chain, or one for all) are replicated over a group's rungs, and
+        ``chain_offset`` (the global id of the first engine chain) must be a multiple of R"""
+        R = 1 if ladder is None else len(ladder)
+        self.R = R
         self.ranges = [shard_range(n_chains, i, len(self)) for i in range(len(self))]
         if any(hi == lo for lo, hi in self.ranges):
             raise ValueError("n_chains must be at least the number of devices")
@@ -70,7 +77,11 @@ class EngineGroup:
         def init(i, e):
             lo, hi = self.ranges[i]
             q = None if q0 is None else (q0[lo:hi] if q0.shape[0] == n_chains else q0)
-            e.hmc_init(hi - lo, eps, m, L, semantics, q0=q, chain_offset=chain_offset + lo)
+            if q is not None and R > 1:
+                q = np.repeat(q.reshape(-1, q.shape[-1]), R, axis=0) if q.shape[0] == hi - lo else q
+            e.hmc_init((hi - lo) * R, eps, m, L, semantics, q0=q, chain_offset=chain_offset + lo * R)
+            if R > 1:
+                e.hmc_set_temperatures(ladder)
         self.each(init)
 
     def hmc_run(self, n, burning, sampling):
@@ -96,10 +107,17 @@ class EngineGroup:
         return np.concatenate(self.each(lambda i, e: e.hmc_step_sizes()))
 
     def hmc_set_step_sizes(self, eps):
+        """one step size per engine chain (n_chains R with a ladder), global chain order"""
         eps = np.asarray(eps, np.float64).reshape(-1)
-        if eps.shape[0] != self.ranges[-1][1]:
-            raise ValueError("expected %d step sizes, got %d" % (self.ranges[-1][1], eps.shape[0]))
-        self.each(lambda i, e: e.hmc_set_step_sizes(eps[self.ranges[i][0]:self.ranges[i][1]]))
+        R = getattr(self, "R", 1)
+        if eps.shape[0] != self.ranges[-1][1] * R:
+            raise ValueError("expected %d step sizes, got %d" % (self.ranges[-1][1] * R, eps.shape[0]))
+        self.each(lambda i, e: e.hmc_set_step_sizes(eps[self.ranges[i][0] * R:self.ranges[i][1] * R]))
+
+    def hmc_tempering_stats(self):
+        """``Engine.hmc_tempering_stats`` of the last ``hmc_run``, summed over the devices"""
+        parts = self.each(lambda i, e: e.hmc_tempering_stats())
+        return {k: sum(p[k] for p in parts) for k in parts[0]}
 
     def hmc_track_predictive(self, x, y=None):
         self.each(lambda i, e: e.hmc_track_predictive(x, y))
@@ -116,7 +134,7 @@ class EngineGroup:
             sums += p[0]
             if s2 is not None:
                 s2 += p[1]
-        n_chains = sum(e.S for e in self.engines)
+        n_chains = sum(e.S // e.R for e in self.engines)       # a ladder tracks its rung-0 chains
         T = Ts.pop()
         return self.engines[0].hmc_predictive_finish(sums, s2, n_chains, T, semantics, divisor), n_chains, T
 

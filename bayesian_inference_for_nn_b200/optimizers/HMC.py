@@ -28,6 +28,17 @@ step sizes are frozen and the k sampling iterations run as before.  Adaptation d
 float64, global chain order; ``epsilon`` everywhere without adaptation).  Chains adapt independently, so a run sharded
 over devices gives the one-device step sizes.
 
+Parallel tempering: ``inverse_temperatures`` (default absent: off), a list of R inverse temperatures starting at 1.0 and
+strictly decreasing to > 0.  Every one of the ``n_chains`` posterior chains then runs as a replica group of R chains
+(``n_chains R`` engine chains; q0 rows are replicated over a group's rungs), rung r sampling prior x likelihood^beta_r,
+and after every iteration neighbouring rungs propose to swap their states (non-reversible even-odd replica exchange,
+Syed et al. 2022), so a cold chain stuck in one mode of the posterior gets states from the hotter rungs, which move
+between modes easily.  Only the beta = 1 rung is a posterior sample: ``result()``, ``predictive()`` and
+``classification_uncertainty()`` see its draws only, and ``accept_rate`` and the progress line report it.
+``tempering_rates()`` gives the per-rung HMC acceptance and per-pair swap acceptance of the sampling phase, the numbers
+to tune a ladder by (a swap rate near 0 between two rungs asks for a rung between them); ``step_sizes`` is then
+[n_chains, R].  The ladder is checked before any device work (``tempering.validate_ladder``).
+
 Streamed predictive: ``track_predictive(x, y=None)`` after ``compile`` and before ``train`` / the first sampling
 ``step`` makes every recorded draw go through the forward pass on x while the chains run.  ``predictive()`` then gives
 what ``result().predict(x, 0, mode="exact")`` and ``last_variance`` give, plus the R-hat of every output across the
@@ -42,6 +53,7 @@ from ..distributions import Sampled
 from ..keras_json import parse_model_json
 from ..multi import EngineGroup, devices_from
 from ..nn import BayesianModel
+from ..tempering import validate_ladder
 from ..tensors import to_numpy
 from .Optimizer import Optimizer
 
@@ -67,6 +79,9 @@ class HMC(Optimizer):
         self._keep_samples = True
         self._adapt_iterations = 0
         self._target_accept = 0.8
+        self._ladder = None
+        self._R = 1
+        self._temper = None
 
     def compile_extra_components(self, **kwargs):
         self._m = self._hyperparameters.m
@@ -89,6 +104,9 @@ class HMC(Optimizer):
             raise ValueError("adapt_iterations must be >= 0")
         if not 0.0 < self._target_accept < 1.0:
             raise ValueError("target_accept must be in (0, 1)")
+        self._ladder = validate_ladder(self._hp("inverse_temperatures", None))
+        self._R = 1 if self._ladder is None else len(self._ladder)
+        self._temper = None
         self._devices = devices_from(self._hp)
         self._engine = EngineGroup(self._spec, self._devices, seed=self.seed)
         path = self._hp("path", "auto")
@@ -104,20 +122,30 @@ class HMC(Optimizer):
                 e.set_option("hmc_keep_samples", 0)
         self._engine.each(setup)
         self._engine.hmc_init(self._n_chains, self._epsilon, self._m, int(self._L), self._semantics,
-                              q0=kwargs.get("q0"), chain_offset=int(self._hp("chain_offset", 0)))
+                              q0=kwargs.get("q0"), chain_offset=int(self._hp("chain_offset", 0)), ladder=self._ladder)
 
     # ---- one iteration (HMC.py:74-104) -----------------------------------------------------
     def step(self, save_document_path=None, sampling=True, burning=False):
         self._sampling_started |= bool(sampling)
         d = self._engine.hmc_run(1, burning=burning, sampling=sampling)
-        self._book(d)
+        self._book(d, sampling)
         return d["mean_loss"]
 
-    def _book(self, d):
+    def _book(self, d, sampling=False):
         self.last_diag = d
-        self._total_runs += d["n_total"]
-        self._accepted_runs += d["n_accepted"]
         self._current_loss = d["mean_loss"]
+        if self._ladder is None:
+            self._total_runs += d["n_total"]
+            self._accepted_runs += d["n_accepted"]
+            return
+        t = self._engine.hmc_tempering_stats()        # the acceptance rate reported is the beta = 1 rung's
+        self._total_runs += int(t["rung_total"][0])
+        self._accepted_runs += int(t["rung_accepted"][0])
+        if sampling:
+            if self._temper is None:
+                self._temper = {k: np.zeros_like(v) for k, v in t.items()}
+            for k, v in t.items():
+                self._temper[k] += v
 
     def _phase(self, n, suffix, sampling, burning):
         """n iterations; with verbose on, the progress line is refreshed ~20 times per phase (each
@@ -127,7 +155,7 @@ class HMC(Optimizer):
         while done < n:
             k = min(chunk, n - done)
             d = self._engine.hmc_run(k, burning=burning, sampling=sampling)
-            self._book(d)
+            self._book(d, sampling)
             done += k
             rate = self._accepted_runs / max(1, self._total_runs)
             self._print_progress(done / n, suffix=suffix, loss=d["mean_loss"], accept_rate=rate, bar_length=20)
@@ -144,6 +172,7 @@ class HMC(Optimizer):
             self._phase(self._adapt_iterations, "HMC - Adapting", sampling=False, burning=False)
             self._engine.hmc_adapt_end()
         self._accepted_runs = self._total_runs = 0
+        self._temper = None
         self._engine.each(lambda i, e: e.hmc_reset_samples())
         self._phase(int(nb_iterations), "HMC - Sampling", sampling=True, burning=False)
 
@@ -153,8 +182,21 @@ class HMC(Optimizer):
 
     @property
     def step_sizes(self):
-        """[n_chains] float64: every chain's step size, in global chain order"""
-        return self._engine.hmc_step_sizes()
+        """[n_chains] float64: every chain's step size, in global chain order; [n_chains, R] (one per rung) with a
+        tempering ladder"""
+        e = self._engine.hmc_step_sizes()
+        return e if self._ladder is None else e.reshape(-1, self._R)
+
+    def tempering_rates(self):
+        """-> (rung_accept [R], swap_accept [R - 1]) float64 over the sampling iterations so far: each rung's HMC
+        acceptance rate and the acceptance rate of the swaps proposed between rungs r and r + 1"""
+        if self._ladder is None:
+            raise RuntimeError("no tempering ladder: set the inverse_temperatures hyper-parameter")
+        t = self._temper
+        if t is None:
+            raise RuntimeError("no sampling iteration has run yet")
+        return (t["rung_accepted"] / np.maximum(1, t["rung_total"]),
+                t["swap_accepted"] / np.maximum(1, t["swap_attempted"]))
 
     # ---- streamed predictive ---------------------------------------------------------------
     def track_predictive(self, x, y=None):
@@ -194,6 +236,7 @@ class HMC(Optimizer):
         samples, freq, _chain = self._engine.hmc_samples()
         if samples.shape[0] == 0:
             q, _ = self._engine.hmc_state()          # no sampling iteration yet: current positions, weight 1
+            q = q[::self._R]                          # (the cold rung of every replica group)
             samples, freq = q, np.ones(q.shape[0], np.int32)
         posterior = BayesianModel(self._model_config, device=self._devices[0])
         posterior.apply_distribution(Sampled(samples, freq.tolist()), 0, self._spec.n_keras_layers - 1)

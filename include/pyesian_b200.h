@@ -105,7 +105,9 @@ int pyb_param_count(const pyb_handle* h, int64_t* n_params_out);
  * of being re-evaluated as HMC.py:80,82 do - L instead of L+1 full-data evaluations per iteration, identical results;
  * "hmc_keep_samples" (default 1): every recorded HMC draw is kept for pyb_hmc_samples; 0 keeps none (no sample arena,
  * no host copy, pyb_hmc_sample_count returns 0) for runs that only need the streamed predictive
- * (pyb_hmc_track_predictive); the chains move identically either way.  It cannot change during a sampling phase. */
+ * (pyb_hmc_track_predictive); the chains move identically either way.  It cannot change during a sampling phase.
+ * "hmc_swap" (default 1): with a tempering ladder set (pyb_hmc_set_temperatures), 0 keeps the ladder but proposes no
+ * replica swaps (the rungs then run side by side as independent tempered chains). */
 int pyb_set_option(pyb_handle* h, const char* key, double value);
 /* read-outs: "path_used", "kernel_launches", "last_device_ms", "workspace_bytes", "tensor_path_ok", "hmc_arena_rows"
  * (rows of the device sample arena, 0 while it has never been sized), "fs_cluster_used" (CTAs per chain of the last
@@ -170,6 +172,45 @@ int pyb_hmc_adapt_begin(pyb_handle* h, double target_accept);
 int pyb_hmc_adapt_end(pyb_handle* h);
 int pyb_hmc_step_sizes(pyb_handle* h, double* eps_out);
 int pyb_hmc_set_step_sizes(pyb_handle* h, const double* eps);
+
+/* ---- parallel tempering: HMC chains as ladders of tempered replicas with replica exchange on the device ----
+ * Ladder.  R >= 2 inverse temperatures beta_0 = 1 > beta_1 > ... > beta_{R-1} > 0 (R <= 64).  Local chain s = g R + r
+ *   is rung r of replica group g: groups are contiguous and group-major, so global chain ids stay chain_offset + s and
+ *   every Philox stream keeps its key.  S and chain_offset must be multiples of R, so a shard always holds whole groups.
+ * Tempered potential.  Chain s samples prior(q) exp(-beta_r E(q)) with E = n_train mean_loss: in float
+ *   U = (Up + prior_const) + (beta_r loss) n_train and dU/dq = beta_r g_data + (q - mu) / sigma^2.  The loss and loss
+ *   gradient carried between iterations ("hmc_carry") stay untempered, so a state keeps its evaluation when it moves to
+ *   another rung.  With beta = 1 every expression rounds exactly as without a ladder: the cold rung moves bit for bit as
+ *   an untempered chain with the same global id (as long as no swap reaches it).
+ * Swap move.  After every iteration's accept / restore, one deterministic even-odd round (Syed, Bouchard-Cote,
+ *   Deligiannidis & Doucet 2022, non-reversible parallel tempering): in iteration iter the pairs (r, r + 1) with
+ *   r = iter (mod 2) of every group propose to exchange their states, accepted iff u < exp(log_r) with
+ *     log_r = (beta_r - beta_{r+1}) n_train ((double)loss_r - (double)loss_{r+1})   in double (NaN rejects),
+ *     u = the Philox uniform of global chain chain_offset + g R + r, iteration iter, stream 4 (seed).
+ *   loss is the untempered mean loss at each chain's current position (pyb_hmc_last's loss).  An accepted swap exchanges
+ *   the two chains' positions, their carried loss gradients and losses; momenta are redrawn every iteration, and step
+ *   sizes and their dual-averaging state stay with the chain slot (each rung adapts its own).  Swaps run in every
+ *   iteration while a ladder is set: burn-in, adaptation and sampling.
+ * Draws.  Only rung-0 chains record draws, into the samples and the tracked predictive: the state before the first
+ *   sampling iteration, then a new draw whenever the position changed (HMC accept or swap; the draw is the position
+ *   after the swap), else the last draw's frequency grows.  pyb_hmc_samples returns them with their global chain ids;
+ *   the tracked predictive keeps sums for the S / R cold chains (n_chains of pyb_hmc_predictive_finish = the number of
+ *   groups).  pyb_hmc_diag still counts all chains.
+ * Sharding.  Groups never straddle handles and swaps never cross them: a sharded run reproduces the unsharded one bit
+ *   for bit with no collective.
+ * pyb_hmc_set_temperatures: beta [R] host float64; beta = NULL with R = 0 turns tempering off.  PYB_ERR_INVALID for a
+ *   ladder outside the rules above; PYB_ERR_STATE before pyb_hmc_init and once a sampling iteration has run since
+ *   pyb_hmc_init / pyb_hmc_reset_samples.  pyb_hmc_init clears the ladder.
+ * pyb_hmc_tempering_stats: host arrays of R, R, R - 1 and R - 1 entries (any may be NULL): per rung the HMC proposals
+ *   accepted and made, per pair (r, r + 1) the swaps attempted and accepted, counted over the last pyb_hmc_run call and
+ *   this handle's groups (counts of different handles add up).  PYB_ERR_STATE without a ladder.
+ * pyb_hmc_last_swaps: per chain [S] the log ratio of the swap proposed with its upper neighbour in the last iteration
+ *   and whether it was taken (NaN and 0 for a chain that proposed none).  PYB_ERR_STATE without a ladder or before an
+ *   iteration has run under it. */
+int pyb_hmc_set_temperatures(pyb_handle* h, const double* beta, int32_t R);
+int pyb_hmc_tempering_stats(pyb_handle* h, int64_t* rung_accepted, int64_t* rung_total, int64_t* swap_attempted,
+                            int64_t* swap_accepted);
+int pyb_hmc_last_swaps(pyb_handle* h, float* log_r, int32_t* swapped);
 
 /* ---- streamed HMC posterior predictive (BayesianModel.predict BayesianModel.py:106-129 in mode "exact" over the draws
  *      HMC records, HMC.py:92-104; Metrics.classification_uncertainty Metrics.py:344-375) ----
