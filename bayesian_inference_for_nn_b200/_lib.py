@@ -74,6 +74,9 @@ SIGNATURES = {
     "pyb_hmc_predictive_sums": [_P, _f64p, _f64p, C.POINTER(C.c_int64)],
     "pyb_hmc_predictive_finish": [_P, _f64p, _f64p, C.c_int64, C.c_int64, C.c_int32, C.c_double, _f32p, _f32p, _f32p,
                                   _f32p, _f32p, _f32p],
+    "pyb_hmc_track_params": [_P, C.c_int64, C.c_int32],
+    "pyb_hmc_param_sums": [_P, _f64p, C.POINTER(C.c_int64)],
+    "pyb_hmc_param_finish": [_P, _f64p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _f64p, _f64p, _f64p, _f64p, _f64p],
     "pyb_svgd_init": [_P, C.c_int64, C.c_int64, C.c_double, C.c_int32, _f64p],
     "pyb_svgd_step": [_P, _i32p, C.c_int64, C.POINTER(C.c_double)],
     "pyb_svgd_phi": [_P, _f64p, _f32p, C.c_int64, C.c_int32, _f32p, C.POINTER(C.c_double)],

@@ -284,6 +284,7 @@ int pyb_get_info(const pyb_handle* h, const char* key, double* out) {
   else if (!strcmp(key, "last_device_ms")) *out = h->last_device_ms;
   else if (!strcmp(key, "sm_count")) *out = h->sm_count;
   else if (!strcmp(key, "fs_cluster_used")) *out = h->fs_cluster_used;
+  else if (!strcmp(key, "hmc_param_bytes")) *out = (double)hmc_params_bytes(h);
   else if (!strcmp(key, "prof_ms")) *out = h->prof_ms;
   else if (!strcmp(key, "prof_flops")) *out = h->prof_flops;
   else if (!strcmp(key, "prof_launches")) *out = (double)h->prof_launches;
@@ -544,6 +545,7 @@ int pyb_hmc_reset_samples(pyb_handle* h) {
   st.host_last_idx.assign(st.S, -1);
   st.sampling_started = false;
   hmc_track_clear(h);
+  hmc_params_clear(h);
   PYB_CATCH
 }
 
@@ -668,6 +670,37 @@ int pyb_hmc_predictive_finish(pyb_handle* h, const double* sums, const double* s
     PYB_REQUIRE(uq_semantics == PYB_UQ_REFERENCE || uq_semantics == PYB_UQ_CANONICAL, PYB_ERR_INVALID, "bad semantics");
   UncertaintyReq uq{nullptr, uq_semantics == PYB_UQ_REFERENCE ? 1 : 0, divisor, total_out, aleatoric_out, epistemic_out};
   hmc_track_finish(h, sums, s2, n_chains, n_draws, want_uq ? &uq : nullptr, mean_out, var_out, rhat_out);
+  PYB_CATCH
+}
+
+int pyb_hmc_track_params(pyb_handle* h, int64_t n_planned, int32_t batch) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  if (n_planned == 0) {
+    PYB_CUDA(cudaStreamSynchronize(h->stream));
+    hmc_params_stop(h);
+  } else {
+    hmc_params_start(h, n_planned, batch);
+  }
+  PYB_CATCH
+}
+
+int pyb_hmc_param_sums(pyb_handle* h, double* sums_out, int64_t* n_draws_out) {
+  PYB_TRY
+  PYB_REQUIRE(h && sums_out, PYB_ERR_INVALID, "NULL argument");
+  use_device(h);
+  hmc_params_sums(h, sums_out, n_draws_out);
+  PYB_CATCH
+}
+
+int pyb_hmc_param_finish(pyb_handle* h, const double* sums, int64_t n_chains, int64_t n_draws, int64_t n_planned,
+                         int32_t batch, double* mean_out, double* sd_out, double* rhat_out, double* ess_out,
+                         double* mcse_out) {
+  PYB_TRY
+  PYB_REQUIRE(h, PYB_ERR_INVALID, "NULL handle");
+  use_device(h);
+  hmc_params_finish(h, sums, n_chains, n_draws, n_planned, batch, mean_out, sd_out, rhat_out, ess_out, mcse_out);
   PYB_CATCH
 }
 

@@ -186,6 +186,23 @@ __device__ inline void dual_average(double* da, double* step, float log_alpha, d
   *step = exp(log_eps);
 }
 
+// classic Gelman-Rubin R-hat of element e from sums over S chains with T draws each: A = sum of all draws,
+// M = sum_s (sum_t x)^2, Wss = within-chain sum of squares sum_s sum_t (x - m_s)^2:
+//   W = Wss / (S (T-1)),  B/T = var_s(m_s) (ddof 1) = (M/T^2 - S mu^2) / (S-1),
+//   V = (T-1)/T W + B/T,  R-hat = sqrt(V / W);  NaN when S < 2, T < 2 or W = 0 (or a sum is NaN)
+__device__ inline double gelman_rubin(const double* A, const double* M, const double* Wss, int64_t e, double S,
+                                      double T) {
+  double r = NAN;
+  if (S >= 2.0 && T >= 2.0) {
+    const double W = Wss[e] / (S * (T - 1.0));
+    const double mu = A[e] / (S * T);
+    double bt = (M[e] / (T * T) - S * mu * mu) / (S - 1.0);
+    if (bt < 0.0) bt = 0.0;
+    if (W > 0.0) r = sqrt(((T - 1.0) / T * W + bt) / W);
+  }
+  return r;
+}
+
 __device__ inline float act_apply(float z, int act) {
   switch (act) {
     case PYB_ACT_RELU: return fmaxf(z, 0.0f);
@@ -267,6 +284,18 @@ struct HmcState {
     DevBuf<double> S2;          // [Nt, C, C] pooled sum o o^T (labels given and C > 1)
     DevBuf<double> part;        // [chain groups, 2, Nt, C] partial sums of one chunk
   } track;
+  // streamed per-parameter moments (hmc_params.cu): the same draws as `track`, in weight space
+  struct ParamTrack {
+    bool on = false;
+    int64_t T = 0;              // draws per chain so far
+    int64_t nch = 0;            // tracked chains: S, or the S / R rung-0 chains of a tempering ladder
+    int64_t n_planned = 0, half = 0, batch = 0;   // h = n_planned / 2 and the batch size b, fixed at the start
+    int ngroups = 0;            // chain groups of the accumulation kernel (a function of nch and P)
+    DevBuf<float> shift;        // [nch, P] each chain's first draw c
+    DevBuf<double> d, hcur, bcur, bsum;   // [nch, P] per chain: sum_t (x - c), the current half's and batch's, sum of batches
+    DevBuf<double> pool;        // [kParamPooled, P] pooled over chains (hmc_params.cu)
+    DevBuf<double> part;        // [ngroups, kParamPooled, P] one draw's group partials
+  } ptrack;
 };
 
 struct SvgdState {
@@ -558,4 +587,15 @@ void hmc_track_resize(pyb_handle* h);
 void hmc_track_sums(pyb_handle* h, double* sums, double* s2, int64_t* n_draws);
 void hmc_track_finish(pyb_handle* h, const double* sums, const double* s2, int64_t n_chains, int64_t n_draws,
                       const UncertaintyReq* uq, float* mean, float* var, float* rhat);
+
+// hmc_params.cu
+void hmc_params_start(pyb_handle* h, int64_t n_planned, int64_t batch);
+void hmc_params_stop(pyb_handle* h);
+void hmc_params_clear(pyb_handle* h);
+void hmc_params_resize(pyb_handle* h);
+void hmc_params_draw(pyb_handle* h);
+void hmc_params_sums(pyb_handle* h, double* sums, int64_t* n_draws);
+void hmc_params_finish(pyb_handle* h, const double* sums, int64_t n_chains, int64_t n_draws, int64_t n_planned,
+                       int64_t batch, double* mean, double* sd, double* rhat, double* ess, double* mcse);
+size_t hmc_params_bytes(const pyb_handle* h);
 }  // namespace pyb

@@ -76,22 +76,12 @@ __global__ void k_track_reduce(const float* __restrict__ shift, const double* __
   W[e] = Qd[e] - dd / T;
 }
 
-// classic Gelman-Rubin R-hat per output element from the sums of S chains with T draws each:
-//   W = (within-chain SS) / (S (T-1)),  B/T = var_s(m_s) (ddof 1) = (M/T^2 - S mu^2) / (S-1),
-//   V = (T-1)/T W + B/T,  R-hat = sqrt(V / W);  NaN when S < 2, T < 2 or W = 0
+// classic Gelman-Rubin R-hat (gelman_rubin, common.cuh) per output element from the sums of S chains with T draws each
 __global__ void k_track_rhat(const double* __restrict__ A, const double* __restrict__ M, const double* __restrict__ Wss,
                              int64_t elems, double S, double T, float* rhat) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= elems) return;
-  double r = NAN;
-  if (S >= 2.0 && T >= 2.0) {
-    const double W = Wss[e] / (S * (T - 1.0));
-    const double mu = A[e] / (S * T);
-    double bt = (M[e] / (T * T) - S * mu * mu) / (S - 1.0);
-    if (bt < 0.0) bt = 0.0;
-    if (W > 0.0) r = sqrt(((T - 1.0) / T * W + bt) / W);
-  }
-  rhat[e] = (float)r;
+  rhat[e] = (float)gelman_rubin(A, M, Wss, e, S, T);
 }
 
 static bool track_tensor(pyb_handle* h, int64_t Nt) {   // the forward pyb_predict would use for these inputs

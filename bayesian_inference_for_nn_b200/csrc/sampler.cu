@@ -435,6 +435,7 @@ void hmc_init(pyb_handle* h, int64_t S, int64_t chain_offset, double eps, double
   st.tcount.release(); st.cold.release();
   st.swaps_ran = false;
   hmc_track_stop(h);
+  hmc_params_stop(h);
   DevBuf<float> tmp;
   const float* q0d = nullptr;
   if (q0) {
@@ -531,10 +532,13 @@ static bool update_i8_guard(pyb_handle* h, const float* loss_dev, int64_t S) {
   return ok;
 }
 
-// one tracked draw of every chain at its current position; a ladder tracks its rung-0 chains, gathered into [G, P]
+// one tracked draw of every chain at its current position; a ladder tracks its rung-0 chains (the parameter sums read
+// them in place, the predictive gathers them into [G, P])
 static void track_current(pyb_handle* h) {
   HmcState& st = h->hmc;
   const int64_t P = h->model.P;
+  if (st.ptrack.on) hmc_params_draw(h);
+  if (!st.track.on) return;
   if (!st.R) { hmc_track_draw(h, st.q.p, st.S); return; }
   const int64_t G = st.S / st.R;
   PYB_CUDA(cudaMemcpy2DAsync(st.cold.p, P * sizeof(float), st.q.p, st.R * P * sizeof(float), P * sizeof(float), G,
@@ -603,7 +607,8 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
       if (st.arena_used_upper + need > st.arena_cap) hmc_flush_arena(h);
       st.arena_used_upper += need;
     }
-    if (first && st.track.on) track_current(h);     // the pre-iteration state is the first draw (HMC.py:75-77)
+    const bool tracking = st.track.on || st.ptrack.on;
+    if (first && tracking) track_current(h);        // the pre-iteration state is the first draw (HMC.py:75-77)
     if (st.adapting) st.adapt_t++;
     dim3 gridp = chain_grid(nblk, S);
     if (path == PYB_PATH_FUSED_SMALL) {
@@ -672,7 +677,7 @@ void hmc_run(pyb_handle* h, int n_iters, bool burning, bool sampling, pyb_hmc_di
     count_launch(h);
     }
     if (sampling) st.sampling_started = true;
-    if (sampling && st.track.on) track_current(h);  // the post-accept (post-swap) position (HMC.py:92-104)
+    if (sampling && tracking) track_current(h);     // the post-accept (post-swap) position (HMC.py:92-104)
     if (carry)     // loss at the new current position = what step() returns: accepted ? loss(q_L) : loss(q0) (HMC.py:96,104)
       PYB_CUDA(cudaMemcpyAsync(st.loss0.p, st.ret_loss.p, S * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
     st.have_cur = carry;
@@ -835,6 +840,7 @@ void hmc_set_temperatures(pyb_handle* h, const double* beta, int R) {
     st.tcount.release(); st.cold.release();
     st.swaps_ran = false;
     hmc_track_resize(h);
+    hmc_params_resize(h);
     return;
   }
   PYB_REQUIRE(beta, PYB_ERR_INVALID, "beta is NULL (pass NULL with R = 0 to turn tempering off)");
@@ -858,6 +864,7 @@ void hmc_set_temperatures(pyb_handle* h, const double* beta, int R) {
   st.R = R;
   st.swaps_ran = false;
   hmc_track_resize(h);
+  hmc_params_resize(h);
 }
 
 void hmc_tempering_stats(pyb_handle* h, int64_t* rung_acc, int64_t* rung_tot, int64_t* swap_att, int64_t* swap_acc) {

@@ -283,6 +283,31 @@ class Engine:
             raise RuntimeError("no predictive is tracked: call hmc_track_predictive first")
         return t
 
+    # ---- streamed per-parameter moments (pyb_hmc_track_params / pyb_hmc_param_sums / pyb_hmc_param_finish)
+    def hmc_track_params(self, n_planned, batch=0):
+        """Accumulate the mean, sd, split-R-hat, ESS and MCSE of every parameter over every draw the sampler records
+        from the next sampling iteration on, planned for ``n_planned`` draws per chain (it fixes the split halves) with
+        batch size ``batch`` (0: floor(sqrt(n_planned))).  n_planned = 0 stops tracking."""
+        check(self.lib.pyb_hmc_track_params(self.h, int(n_planned), int(batch)))
+
+    def hmc_param_sums(self):
+        """-> (sums [7, P] float64 = A, M, W, Ah, Mh, Wh, V, draws per chain T)"""
+        sums = np.empty((7, self.P), np.float64)
+        T = C.c_int64()
+        check(self.lib.pyb_hmc_param_sums(self.h, _ptr(sums), C.byref(T)))
+        return sums, T.value
+
+    def hmc_param_finish(self, sums, n_chains, n_draws, n_planned, batch=0):
+        """-> dict of mean, sd, rhat (split), ess, mcse, each [P] float64, from (summed) ``hmc_param_sums``"""
+        sums = np.ascontiguousarray(sums, dtype=np.float64)
+        if sums.shape != (7, self.P):
+            raise ValueError("sums must be [7, %d]" % self.P)
+        out = {k: np.empty(self.P, np.float64) for k in ("mean", "sd", "rhat", "ess", "mcse")}
+        check(self.lib.pyb_hmc_param_finish(self.h, _ptr(sums), int(n_chains), int(n_draws), int(n_planned), int(batch),
+                                            _ptr(out["mean"]), _ptr(out["sd"]), _ptr(out["rhat"]), _ptr(out["ess"]),
+                                            _ptr(out["mcse"])))
+        return out
+
     # ---- SVGD
     def svgd_init(self, S, lr, semantics=_lib.SVGD_REFERENCE_LIVE, particles0=None, offset=0):
         p0 = None if particles0 is None else np.ascontiguousarray(particles0, dtype=np.float64)

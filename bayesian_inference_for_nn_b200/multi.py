@@ -138,6 +138,23 @@ class EngineGroup:
         T = Ts.pop()
         return self.engines[0].hmc_predictive_finish(sums, s2, n_chains, T, semantics, divisor), n_chains, T
 
+    def hmc_track_params(self, n_planned, batch=0):
+        self.each(lambda i, e: e.hmc_track_params(n_planned, batch))
+
+    def hmc_param_summary(self, n_planned, batch=0):
+        """the streamed per-parameter moments over every device's chains: the per-device sums are added on the host in
+        device order and finished on engine 0 -> (``hmc_param_finish`` dict, n_chains, T)"""
+        parts = self.each(lambda i, e: e.hmc_param_sums())
+        Ts = {p[1] for p in parts}
+        if len(Ts) != 1:
+            raise RuntimeError("the devices tracked different numbers of draws per chain: %s" % sorted(Ts))
+        sums = parts[0][0].copy()
+        for p in parts[1:]:
+            sums += p[0]
+        n_chains = sum(e.S // e.R for e in self.engines)       # a ladder tracks its rung-0 chains
+        T = Ts.pop()
+        return self.engines[0].hmc_param_finish(sums, n_chains, T, n_planned, batch), n_chains, T
+
     # ---- SVGD -----------------------------------------------------------------------------------------------------
     def svgd_join(self):
         """one NCCL communicator over the group's engines (a no-op for one device)"""

@@ -43,6 +43,16 @@ Streamed predictive: ``track_predictive(x, y=None)`` after ``compile`` and befor
 ``step`` makes every recorded draw go through the forward pass on x while the chains run.  ``predictive()`` then gives
 what ``result().predict(x, 0, mode="exact")`` and ``last_variance`` give, plus the R-hat of every output across the
 chains; ``classification_uncertainty`` what ``result().classification_uncertainty(x, y, 0, mode="exact")`` gives.
+
+Streamed parameter diagnostics: ``track_parameters(n_iterations=None, batch_size=None)`` after ``compile`` folds every
+parameter of every recorded draw into sums on the device, so it works with ``keep_samples=False`` too.
+``parameter_summary()`` then gives, per parameter in the flat weight order, the posterior mean and sd (what the
+frequency-weighted ``result()`` samples give), the split R-hat over half-chains (Gelman et al., BDA3 11.4; it flags a
+chain that drifts, which the classic R-hat misses), the batch-means effective sample size (Flegal & Jones 2010) and the
+Monte Carlo standard error of the mean, with the number of chains and draws per chain.  ``train(n)`` plans the halves for
+its n + 1 draws per chain; without ``train``, ``n_iterations`` (the sampling iterations to come) is required and the
+tracking starts at once.  ``batch_size`` defaults to floor(sqrt(draws)).  ESS per gradient evaluation is the number to
+tune epsilon, L, ``target_accept`` or a ladder by.
 """
 from collections import namedtuple
 
@@ -58,6 +68,7 @@ from ..tensors import to_numpy
 from .Optimizer import Optimizer
 
 Predictive = namedtuple("Predictive", ["mean", "variance", "rhat", "n_chains", "n_draws"])
+ParameterSummary = namedtuple("ParameterSummary", ["mean", "sd", "rhat", "ess", "mcse", "n_chains", "n_draws"])
 
 _PATHS = {"auto": _lib.PATH_AUTO, "generic": _lib.PATH_GENERIC, "fused": _lib.PATH_FUSED_SMALL,
           "tensor": _lib.PATH_TENSOR}
@@ -76,6 +87,7 @@ class HMC(Optimizer):
         self.last_diag = None
         self._sampling_started = False
         self._tracking = False
+        self._ptrack = None              # track_parameters: {"batch": b, "n_planned": draws per chain or None}
         self._keep_samples = True
         self._adapt_iterations = 0
         self._target_accept = 0.8
@@ -174,6 +186,9 @@ class HMC(Optimizer):
         self._accepted_runs = self._total_runs = 0
         self._temper = None
         self._engine.each(lambda i, e: e.hmc_reset_samples())
+        if self._ptrack is not None:
+            self._ptrack["n_planned"] = int(nb_iterations) + 1
+            self._engine.hmc_track_params(self._ptrack["n_planned"], self._ptrack["batch"])
         self._phase(int(nb_iterations), "HMC - Sampling", sampling=True, burning=False)
 
     @property
@@ -228,6 +243,35 @@ class HMC(Optimizer):
         given to ``track_predictive``."""
         r, _, _ = self._tracked(semantics, divisor)
         return r["total"], r["aleatoric"], r["epistemic"]
+
+    # ---- streamed parameter diagnostics ----------------------------------------------------
+    def track_parameters(self, n_iterations=None, batch_size=None):
+        """Track the per-parameter posterior moments and convergence diagnostics over every draw the chains record.
+        Call after ``compile`` and before ``train`` or the first sampling ``step``.  ``train(n)`` plans for its n + 1
+        draws per chain; for sampling by ``step``, ``n_iterations`` (the sampling iterations to come) is required and
+        the tracking starts now.  ``batch_size``: draws per batch of the ESS (default floor(sqrt(draws)))."""
+        if self._engine is None:
+            raise RuntimeError("compile the optimizer before tracking the parameters")
+        if self._sampling_started:
+            raise RuntimeError("track_parameters must be called before train() / the first sampling step")
+        if batch_size is not None and int(batch_size) < 1:
+            raise ValueError("batch_size must be >= 1")
+        self._ptrack = {"batch": 0 if batch_size is None else int(batch_size), "n_planned": None}
+        if n_iterations is not None:
+            self._ptrack["n_planned"] = int(n_iterations) + 1
+            self._engine.hmc_track_params(self._ptrack["n_planned"], self._ptrack["batch"])
+
+    def parameter_summary(self) -> ParameterSummary:
+        """-> (mean, sd, rhat, ess, mcse, n_chains, n_draws): per parameter ([P] float64, flat weight order) the mean
+        and population sd over every recorded draw, the split R-hat, the batch-means effective sample size and the
+        Monte Carlo standard error of the mean.  NaN marks a diverged chain, or a diagnostic that the draws do not
+        define (too few draws or batches, or chains that never moved)."""
+        t = self._ptrack
+        if t is None or t["n_planned"] is None:
+            raise RuntimeError("no parameters are tracked: call track_parameters() before train(), or "
+                               "track_parameters(n_iterations) before sampling by step()")
+        r, n_chains, T = self._engine.hmc_param_summary(t["n_planned"], t["batch"])
+        return ParameterSummary(r["mean"], r["sd"], r["rhat"], r["ess"], r["mcse"], n_chains, T)
 
     def result(self) -> BayesianModel:
         if not self._keep_samples:

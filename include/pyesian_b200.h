@@ -111,7 +111,8 @@ int pyb_param_count(const pyb_handle* h, int64_t* n_params_out);
 int pyb_set_option(pyb_handle* h, const char* key, double value);
 /* read-outs: "path_used", "kernel_launches", "last_device_ms", "workspace_bytes", "tensor_path_ok", "hmc_arena_rows"
  * (rows of the device sample arena, 0 while it has never been sized), "fs_cluster_used" (CTAs per chain of the last
- * small-width HMC launch: 1, 2, 4 or 8; 0 before the first) */
+ * small-width HMC launch: 1, 2, 4 or 8; 0 before the first), "hmc_param_bytes" (device bytes held by
+ * pyb_hmc_track_params) */
 int pyb_get_info(const pyb_handle* h, const char* key, double* value_out);
 
 /* ---- inputs ---- */
@@ -239,6 +240,44 @@ int pyb_hmc_predictive_sums(pyb_handle* h, double* sums_out, double* s2_out, int
 int pyb_hmc_predictive_finish(pyb_handle* h, const double* sums, const double* s2, int64_t n_chains, int64_t n_draws,
                               int32_t uq_semantics, double divisor, float* mean_out, float* var_out, float* rhat_out,
                               float* total_out, float* aleatoric_out, float* epistemic_out);
+
+/* ---- streamed per-parameter posterior moments and convergence diagnostics of the HMC chains ----
+ * The tracked draws are those of the streamed predictive (and of pyb_hmc_samples with their frequencies): the state
+ * before the first sampling iteration after pyb_hmc_init / pyb_hmc_reset_samples, then the position after every
+ * sampling iteration (after accept / restore and the swap round); with a ladder the S / R rung-0 chains only.  So every
+ * tracked chain has the same number T of draws; after n sampling iterations T = n + 1.  Every parameter (flat order of
+ * the weight layout) of every draw is folded into sums inside pyb_hmc_run; nothing is mapped: a NaN parameter (a
+ * diverged chain) gives NaN results.
+ * Definitions, with S chains, T draws x_st each, h = floor(n_planned / 2), the batch size b and a = floor(T / b):
+ *   mean = sum x / (S T);  sd = sqrt of the population variance over all S T draws (pyb_predict's weighting).
+ *   split-R-hat = the classic R-hat (pyb_hmc_predictive_finish) over the 2 S half-chains [0, h) and [h, 2h) of h draws;
+ *     draws from 2h on count in the moments and the ESS only.  NaN when T < 2h, h < 2 or the within-chain variance is 0.
+ *   ESS by batch means (Flegal & Jones 2010): lambda^2 = W / (S (T - 1)) with W the within-chain sum of squares;
+ *     sigma^2_bm = b V / (S (a - 1)), V = sum_s sum_{k<a} (Ybar_sk - Ybar_s)^2 over the means Ybar_sk of the complete
+ *     batches of chain s and their mean Ybar_s (a trailing partial batch is left out);  ess = S T lambda^2 / sigma^2_bm,
+ *     NaN when T < 2, a < 2, lambda^2 = 0 or sigma^2_bm = 0, and not capped at S T (antithetic chains exceed it).
+ *   mcse = sqrt(sigma^2_bm / (S T))  (NaN when a < 2).
+ * pyb_hmc_track_params: track from the next sampling iteration on, planned for n_planned draws per chain (it fixes h;
+ *   more draws may follow) with batch size b = batch, or floor(sqrt(n_planned)) for batch = 0.  PYB_ERR_STATE before
+ *   pyb_hmc_init and once a sampling iteration has run (until pyb_hmc_reset_samples); PYB_ERR_INVALID for n_planned < 4,
+ *   batch < 0 or fewer than two batches in n_planned.  n_planned = 0 stops tracking and frees its memory.  Device
+ *   memory: 36 bytes per (tracked chain, parameter) plus 48 P bytes for the pooled sums and 48 P per group of >= 32
+ *   chains of the accumulation, checked up front (PYB_ERR_OOM with
+ *   the size in the message; read back with pyb_get_info "hmc_param_bytes").  pyb_hmc_reset_samples clears the sums,
+ *   pyb_hmc_init stops tracking, and setting or clearing a ladder resizes them to the tracked chains.  The sums are
+ *   added in a fixed order: deterministic, and one call of n iterations gives those of n calls of one.
+ * pyb_hmc_param_sums: sums_out [7, P] float64 over this handle's chains, in this order: A = sum of all draws,
+ *   M = sum_s (sum_t x)^2, W = within-chain sum of squares; the same three over the complete half-chains (Ah, Mh, Wh);
+ *   V (above); n_draws_out = T.  All are sums over chains: the sums of handles holding disjoint chains add up.
+ *   PYB_ERR_STATE without tracking or before the first tracked draw.
+ * pyb_hmc_param_finish: from sums (of this handle, or of several added) over n_chains chains with n_draws draws each and
+ *   the n_planned / batch of the tracking: mean_out, sd_out, rhat_out (split), ess_out, mcse_out, each [P] float64 (any
+ *   may be NULL).  PYB_ERR_INVALID for a NULL sums, n_chains or n_draws <= 0, and the n_planned / batch rules above. */
+int pyb_hmc_track_params(pyb_handle* h, int64_t n_planned, int32_t batch);
+int pyb_hmc_param_sums(pyb_handle* h, double* sums_out, int64_t* n_draws_out);
+int pyb_hmc_param_finish(pyb_handle* h, const double* sums, int64_t n_chains, int64_t n_draws, int64_t n_planned,
+                         int32_t batch, double* mean_out, double* sd_out, double* rhat_out, double* ess_out,
+                         double* mcse_out);
 
 /* ---- SVGD (SVGD.py:219-228 compile, :143-157 init, :84-141 step, :54-68 + :183-202 live kernel,
  *      :165-181 median-heuristic kernel, legacy Adam created :226 applied :120) ---- */
