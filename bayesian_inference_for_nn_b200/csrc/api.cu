@@ -284,6 +284,7 @@ int pyb_get_info(const pyb_handle* h, const char* key, double* out) {
   else if (!strcmp(key, "last_device_ms")) *out = h->last_device_ms;
   else if (!strcmp(key, "sm_count")) *out = h->sm_count;
   else if (!strcmp(key, "fs_cluster_used")) *out = h->fs_cluster_used;
+  else if (!strcmp(key, "svgd_stein_used")) *out = h->svgd_stein_used;
   else if (!strcmp(key, "hmc_param_bytes")) *out = (double)hmc_params_bytes(h);
   else if (!strcmp(key, "prof_ms")) *out = h->prof_ms;
   else if (!strcmp(key, "prof_flops")) *out = h->prof_flops;

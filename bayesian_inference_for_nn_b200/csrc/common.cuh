@@ -311,6 +311,7 @@ struct SvgdState {
   // tensor-core Gram / Stein contraction operands (bf16 hi/lo kept as raw 16-bit words)
   DevBuf<uint16_t> xh, xl, yth, ytl, kh, kl;
   DevBuf<float> gram, ybuf, kf, norms;
+  DevBuf<float> center;   // tensor path: per-parameter mean of the particles, subtracted before the Gram and Stein terms
   DevBuf<float> Xb;
   DevBuf<int32_t> yb_i, idx;
   DevBuf<float> yb_f;
@@ -433,6 +434,7 @@ struct pyb_handle {
   int64_t opt_chain_batch = 0;
   int path_used = PYB_PATH_GENERIC;
   int fs_cluster_used = 0;  // CTAs per chain of the last small-width HMC launch (0 before the first)
+  int svgd_stein_used = 0;  // Stein-update branch of the last svgd_step / canonical svgd_phi (SteinBranch in svgd.cu)
   int64_t kernel_launches = 0;
   double last_device_ms = 0;
   pyb::Workspace ws;
@@ -505,7 +507,9 @@ void tc_forward(pyb_handle* h, const float* theta, int64_t S, const float* x, in
 void tc_forward_tracked(pyb_handle* h, const float* theta, int64_t S, const float* x, int64_t N, float* out);
 void tc_invalidate_track(pyb_handle* h);
 void gather_rows_f32(pyb_handle* h, const float* src, const int64_t* idx_host, int64_t n, int64_t row_len, float* dst);
-void tc_split_rows(pyb_handle* h, const float* src, int64_t R, int C, int64_t lds, void* hi, void* lo, int64_t ldd);
+// center != nullptr: column c is split as src - center[c]
+void tc_split_rows(pyb_handle* h, const float* src, int64_t R, int C, int64_t lds, void* hi, void* lo, int64_t ldd,
+                   const float* center = nullptr);
 void tc_split_transpose(pyb_handle* h, const float* src, int R, int C, int64_t lds, void* hi, void* lo, int64_t ldd);
 void tc_gemm_split(pyb_handle* h, const void* a_hi, const void* a_lo, int64_t lda, int64_t a_rows_total, int a_row0, int M,
                    const void* b_hi, const void* b_lo, int64_t ldb, int Nn, int64_t K, float* out, int64_t ldc);

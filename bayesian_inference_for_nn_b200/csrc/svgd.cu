@@ -22,6 +22,9 @@
 
 namespace pyb {
 
+// the Stein-update branch that ran last (info "svgd_stein_used")
+enum SteinBranch { STEIN_LIVE_LAUNCHES = 0, STEIN_LIVE_COOP = 1, STEIN_LIVE_CTA = 2, STEIN_F64 = 3, STEIN_TENSOR = 4, STEIN_PSHARD = 5 };
+
 __global__ void k_svgd_init(float* theta, const double* p0, const float* mu, const float* sigma, int64_t P,
                             uint64_t seed, int64_t offset) {
   int64_t s = blockIdx.y;
@@ -526,11 +529,33 @@ __global__ void __launch_bounds__(256) k_phi_live_all(const double* K, const flo
 }
 
 // ---- tensor-core variant of the canonical update (large S): Gram and K*Y as bf16x3 GEMMs ---------
-__global__ void k_row_norms(const float* X, int64_t P, double* norms) {
+// The particles enter the Gram matrix, the norms and the Stein term X/h2 as x - c, c = their mean over the St rows: d2 and
+// phi are translation-invariant, but d2 = n_i + n_j - 2 G_ij and K (X/h2) - X_i rowsum_i/h2 cancel to O((|c|/spread)^2)
+// of the fp32 / bf16x3 rounding when the particles sit close together far from the origin.
+// c[p] = mean over the R rows of column p of X [R, C] (row pitch C), summed in float64 in a fixed order; grid ceil(C/32),
+// block (32, 8)
+__global__ void k_col_mean(const float* __restrict__ X, int R, int64_t C, float* __restrict__ c) {
+  __shared__ double part[8][32];
+  const int64_t col = (int64_t)blockIdx.x * 32 + threadIdx.x;
+  double a = 0.0;
+  if (col < C)
+    for (int r = threadIdx.y; r < R; r += 8) a += (double)X[(int64_t)r * C + col];
+  part[threadIdx.y][threadIdx.x] = a;
+  __syncthreads();
+  if (threadIdx.y == 0 && col < C) {
+    for (int k = 1; k < 8; ++k) a += part[k][threadIdx.x];
+    c[col] = (float)(a / (double)R);
+  }
+}
+// squared norms of the centred rows
+__global__ void k_row_norms(const float* X, int64_t P, const float* __restrict__ center, double* norms) {
   __shared__ double scratch[32];
   const float* x = X + (int64_t)blockIdx.x * P;
   double a = 0.0;
-  for (int64_t e = threadIdx.x; e < P; e += blockDim.x) a += (double)x[e] * (double)x[e];
+  for (int64_t e = threadIdx.x; e < P; e += blockDim.x) {
+    const double d = (double)(x[e] - center[e]);
+    a += d * d;
+  }
   double t = block_sum<double>(a, scratch);
   if (threadIdx.x == 0) norms[blockIdx.x] = t;
 }
@@ -567,13 +592,14 @@ __global__ void k_stein_rhs(const float* X, const float* G, const double* h2, in
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
     Y[i] = G[i] - X[i] * inv;
 }
-// phi = (KY + X_i rowsum_i / h2) / St   in place on the GEMM output (fp32: the GEMM output already is)
-__global__ void k_phi_finish(float* phi, const float* X, int64_t P, int r0, int St, const double* h2, const double* rowsum) {
+// phi = (KY + (X_i - c) rowsum_i / h2) / St   in place on the GEMM output (fp32: the GEMM output already is)
+__global__ void k_phi_finish(float* phi, const float* X, int64_t P, int r0, int St, const double* h2, const double* rowsum,
+                             const float* __restrict__ center) {
   const int i = blockIdx.y;
   const float c = (float)(rowsum[i] / h2[0]), inv = 1.0f / (float)St;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < P; e += (int64_t)gridDim.x * blockDim.x) {
     int64_t o = (int64_t)i * P + e;
-    phi[o] = fmaf(X[(int64_t)(r0 + i) * P + e], c, phi[o]) * inv;
+    phi[o] = fmaf(X[(int64_t)(r0 + i) * P + e] - center[e], c, phi[o]) * inv;
   }
 }
 // the same followed by the Adam ascent step on the local particles (theta_local = rows [r0, r0+Sl) of X): one pass
@@ -581,10 +607,12 @@ __global__ void k_phi_finish(float* phi, const float* X, int64_t P, int r0, int 
 __device__ inline float adam_update(float th, float g, float& m, float& v, float lr_t, float b1, float b2, float eh);
 // Flat [Sl*P] indexing: a thread's four elements are one 16-byte access per stream (7 streams: ky, theta, m, v read;
 // theta, m, v written) whatever P is; they may straddle two particle rows, so the row constant is looked up per element.
+// The Stein term uses the centred particle theta - center[e]; the Adam step is applied to theta itself.
 __global__ void __launch_bounds__(256) k_phi_finish_adam(const float* __restrict__ ky, float* __restrict__ theta_local,
                                                          float* __restrict__ am, float* __restrict__ av, int64_t P,
                                                          int64_t total, int St, const double* __restrict__ h2,
-                                                         const double* __restrict__ rowsum, float lr_t) {
+                                                         const double* __restrict__ rowsum,
+                                                         const float* __restrict__ center, float lr_t) {
   const int64_t base = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 4;
   if (base >= total) return;
   const float inv = 1.0f / (float)St;
@@ -601,7 +629,7 @@ __global__ void __launch_bounds__(256) k_phi_finish_adam(const float* __restrict
     float mm[4] = {m4.x, m4.y, m4.z, m4.w}, vv[4] = {v4.x, v4.y, v4.z, v4.w};
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      const float phi = fmaf(tt[j], c, kk[j]) * inv;
+      const float phi = fmaf(tt[j] - center[e], c, kk[j]) * inv;
       tt[j] = adam_update(tt[j], -phi, mm[j], vv[j], lr_t, 0.9f, 0.999f, 1e-7f);
       if (++e == P) { e = 0; ++i; if (j < 3) c = (float)(rowsum[i] * ih2); }
     }
@@ -611,27 +639,29 @@ __global__ void __launch_bounds__(256) k_phi_finish_adam(const float* __restrict
   } else {
     for (int64_t o = base; o < total; ++o) {
       const float th = theta_local[o];
-      const float phi = fmaf(th, c, ky[o]) * inv;
+      const float phi = fmaf(th - center[e], c, ky[o]) * inv;
       theta_local[o] = adam_update(th, -phi, am[o], av[o], lr_t, 0.9f, 0.999f, 1e-7f);
       if (++e == P) { e = 0; ++i; if (o + 1 < total) c = (float)(rowsum[i] * ih2); }
     }
   }
 }
 
-// Y^T = (G - X/h2)^T split into bf16 hi/lo [P, St] (K-major operand of the K*Y GEMM) in one pass.
+// Y^T = (G - (X - c)/h2)^T split into bf16 hi/lo [P, St] (K-major operand of the K*Y GEMM) in one pass.
 // mu != nullptr: G holds the raw scaled loss gradient and the log-posterior gradient is formed here,
 // G_eff = -(G + (X - mu) inv_var) — the separate k_glogp pass (one more read and write of [St, P]) goes away.
 // grid (ceil(P/32), ceil(St/64)), block (32, 8): a warp stores 64 particles x 2 bytes = one 128-byte line per parameter
 __global__ void k_stein_rhs_split_t(const float* __restrict__ X, const float* __restrict__ G, const double* h2, int St,
                                     int64_t P, uint16_t* __restrict__ hi, uint16_t* __restrict__ lo, int64_t ldd,
-                                    const float* __restrict__ mu, const float* __restrict__ inv_var) {
+                                    const float* __restrict__ mu, const float* __restrict__ inv_var,
+                                    const float* __restrict__ center) {
   __shared__ float tile[64][33];
   const float inv = (float)(1.0 / h2[0]);
   const int64_t c0 = (int64_t)blockIdx.x * 32;
   const int r0 = blockIdx.y * 64;
   const int64_t c = c0 + threadIdx.x;
-  float m = 0.f, iv = 0.f;
+  float m = 0.f, iv = 0.f, cc = 0.f;
   if (mu && c < P) { m = mu[c]; iv = inv_var[c]; }
+  if (c < P) cc = center[c];
 #pragma unroll
   for (int i = threadIdx.y; i < 64; i += 8) {
     const int r = r0 + i;
@@ -640,7 +670,7 @@ __global__ void k_stein_rhs_split_t(const float* __restrict__ X, const float* __
       const float x = X[(int64_t)r * P + c];
       float g = G[(int64_t)r * P + c];
       if (mu) g = -(g + (x - m) * iv);
-      v = g - x * inv;
+      v = g - (x - cc) * inv;
     }
     tile[i][threadIdx.x] = v;
   }
@@ -815,16 +845,20 @@ static void phi_canonical(pyb_handle* h, const float* X_all, const float* G_all,
   const int64_t Ppad = (P + 7) / 8 * 8;
   if (tensor) {
     sv.xh.alloc((size_t)St * Ppad); sv.xl.alloc((size_t)St * Ppad);
-    sv.gram.alloc((size_t)Sl * St); sv.norms.alloc(0); sc.Krow.alloc(St);
-    tc_split_rows(h, X_all, St, (int)P, P, sv.xh.p, sv.xl.p, Ppad);
+    sv.gram.alloc((size_t)Sl * St); sv.norms.alloc(0); sc.Krow.alloc(St); sv.center.alloc(P);
+    // every rank holds the same X_all, so every rank computes the same centre
+    k_col_mean<<<(unsigned)((P + 31) / 32), dim3(32, 8), 0, h->stream>>>(X_all, St, P, sv.center.p);
+    tc_split_rows(h, X_all, St, (int)P, P, sv.xh.p, sv.xl.p, Ppad, sv.center.p);
     tc_gemm_split(h, sv.xh.p, sv.xl.p, Ppad, St, r0, Sl, sv.xh.p, sv.xl.p, Ppad, St, P, sv.gram.p, St);
-    k_row_norms<<<St, 256, 0, h->stream>>>(X_all, P, sc.Krow.p);
+    k_row_norms<<<St, 256, 0, h->stream>>>(X_all, P, sv.center.p, sc.Krow.p);
     k_d2_from_gram<<<(unsigned)(((int64_t)Sl * St + 255) / 256), 256, 0, h->stream>>>(sv.gram.p, sc.Krow.p, r0, Sl, St, sv.d2.p);
-    count_launch(h, 2);
+    count_launch(h, 3);
+    h->svgd_stein_used = STEIN_TENSOR;
   } else {
     dim3 g1((St + 15) / 16, (Sl + 15) / 16);
     k_gram_d2<<<g1, 256, 0, h->stream>>>(X_all, P, r0, Sl, St, sv.d2.p);
     count_launch(h);
+    h->svgd_stein_used = STEIN_F64;
   }
   median_bandwidth(h, sv.d2.p, (int64_t)Sl * St, (int64_t)St * St, St, sc.h2.p);
   k_kernel_rowsum<<<Sl, 256, 0, h->stream>>>(sv.d2.p, St, sc.h2.p, sv.rowsum.p);
@@ -839,14 +873,16 @@ static void phi_canonical(pyb_handle* h, const float* X_all, const float* G_all,
     tc_split_rows(h, sv.kf.p, Sl, St, St, sv.kh.p, sv.kl.p, St);
     dim3 gt((unsigned)((P + 31) / 32), (unsigned)((St + 63) / 64)), bt(32, 8);
     k_stein_rhs_split_t<<<gt, bt, 0, h->stream>>>(X_all, G_all, sc.h2.p, St, P, sv.yth.p, sv.ytl.p, St,
-                                                 raw_loss_grad ? h->mu.p : nullptr, raw_loss_grad ? h->inv_var.p : nullptr);
+                                                 raw_loss_grad ? h->mu.p : nullptr, raw_loss_grad ? h->inv_var.p : nullptr,
+                                                 sv.center.p);
     tc_gemm_split(h, sv.kh.p, sv.kl.p, St, Sl, 0, Sl, sv.yth.p, sv.ytl.p, St, (int)P, St, phi_local, P);
     dim3 gf((unsigned)std::min<int64_t>((P + 255) / 256, 1024), (unsigned)Sl);
     if (adam)
       k_phi_finish_adam<<<(unsigned)(((int64_t)Sl * P + 1023) / 1024), 256, 0, h->stream>>>(
-          phi_local, adam->theta_local, adam->am, adam->av, P, (int64_t)Sl * P, St, sc.h2.p, sv.rowsum.p, adam->lr_t);
+          phi_local, adam->theta_local, adam->am, adam->av, P, (int64_t)Sl * P, St, sc.h2.p, sv.rowsum.p, sv.center.p,
+          adam->lr_t);
     else
-      k_phi_finish<<<gf, 256, 0, h->stream>>>(phi_local, X_all, P, r0, St, sc.h2.p, sv.rowsum.p);
+      k_phi_finish<<<gf, 256, 0, h->stream>>>(phi_local, X_all, P, r0, St, sc.h2.p, sv.rowsum.p, sv.center.p);
     count_launch(h, 3);
   } else {
     dim3 g2((unsigned)((P + 255) / 256), (Sl + 7) / 8);
@@ -1121,11 +1157,14 @@ static void svgd_step_pshard(pyb_handle* h, const float* Xb, const int32_t* yb_i
   sv.xh.alloc((size_t)St * Pw); sv.xl.alloc((size_t)St * Pw);
   sv.gram.alloc((size_t)St * St); sv.d2.alloc((size_t)St * St); sv.rowsum.alloc(St); sv.h2.alloc(2);
   sv.kf.alloc((size_t)St * St); sv.kh.alloc((size_t)St * St); sv.kl.alloc((size_t)St * St);
-  sv.yth.alloc((size_t)Pw * St); sv.ytl.alloc((size_t)Pw * St);
-  tc_split_rows(h, sv.ps_x.p, St, (int)Pw, Pw, sv.xh.p, sv.xl.p, Pw);
+  sv.yth.alloc((size_t)Pw * St); sv.ytl.alloc((size_t)Pw * St); sv.center.alloc(Pw);
+  // the rank's own column slice is centred on its own column means: the Gram matrix is a sum over column slices of
+  // translation-invariant parts, so no collective is needed
+  k_col_mean<<<(unsigned)((Pw + 31) / 32), dim3(32, 8), 0, h->stream>>>(sv.ps_x.p, St, Pw, sv.center.p);
+  tc_split_rows(h, sv.ps_x.p, St, (int)Pw, Pw, sv.xh.p, sv.xl.p, Pw, sv.center.p);
   tc_gemm_split(h, sv.xh.p, sv.xl.p, Pw, St, 0, St, sv.xh.p, sv.xl.p, Pw, St, Pw, sv.gram.p, St);
-  k_row_norms<<<St, 256, 0, h->stream>>>(sv.ps_x.p, Pw, sv.ps_norms.p);
-  count_launch(h);
+  k_row_norms<<<St, 256, 0, h->stream>>>(sv.ps_x.p, Pw, sv.center.p, sv.ps_norms.p);
+  count_launch(h, 2);
   nvtxRangePop();
   mark(1);
   // ---- 2. side stream, third communicator: all-reduce of the Gram matrix, distances, median bandwidth, kernel matrix and
@@ -1212,7 +1251,7 @@ static void svgd_step_pshard(pyb_handle* h, const float* Xb, const int32_t* yb_i
   nvtxRangePushA("pyb.svgd.stein_update(KY+Adam, blocks leave as they finish)");
   dim3 gt((unsigned)((Pw + 31) / 32), (unsigned)((St + 63) / 64)), bt(32, 8);
   k_stein_rhs_split_t<<<gt, bt, 0, h->stream>>>(sv.ps_x.p, sv.ps_g.p, sv.h2.p, St, Pw, sv.yth.p, sv.ytl.p, St, sv.ps_mu.p,
-                                               sv.ps_iv.p);
+                                               sv.ps_iv.p, sv.center.p);
   count_launch(h);
   // remote blocks in the first group: what is left for the second (at most two remote blocks and the own one) is all
   // that can stay exposed after the last multiplication
@@ -1231,7 +1270,7 @@ static void svgd_step_pshard(pyb_handle* h, const float* Xb, const int32_t* yb_i
       tc_gemm_split(h, sv.kh.p, sv.kl.p, St, St, (int)m0, (int)mrows, sv.yth.p, sv.ytl.p, St, (int)Pw, St, sv.ps_phi.p + m0 * Pw, Pw);
       k_phi_finish_adam<<<(unsigned)((mrows * Pw + 1023) / 1024), 256, 0, h->stream>>>(
           sv.ps_phi.p + m0 * Pw, sv.ps_x.p + m0 * Pw, sv.ps_m.p + m0 * Pw, sv.ps_v.p + m0 * Pw, Pw, mrows * Pw, St, sv.h2.p,
-          sv.rowsum.p + m0, lr_t);
+          sv.rowsum.p + m0, sv.center.p, lr_t);
       count_launch(h);
       j += len;
     }
@@ -1332,7 +1371,10 @@ void svgd_step(pyb_handle* h, const int32_t* idx, int64_t B, double* loss_out) {
     nccl_all_gather_f32(sv.nccl_comm, sv.theta.p, sv.theta_all.p, (size_t)S * P, sv.comm_stream);
     PYB_CUDA(cudaEventRecord(sv.ev_theta, sv.comm_stream));
   }
-  if (pshard) svgd_step_pshard(h, Xb, yb_i, yb_f, Nb, lr_t, scale);
+  if (pshard) {
+    svgd_step_pshard(h, Xb, yb_i, yb_f, Nb, lr_t, scale);
+    h->svgd_stein_used = STEIN_PSHARD;
+  }
   else eval_on_batch(h, sv.theta.p, S, Xb, yb_i, yb_f, Nb, scale, sv.loss.p, sv.g.p);
   const bool fold_prior = sv.semantics != PYB_SVGD_REFERENCE_LIVE && svgd_tensor_ok(h, St);
   if (sv.semantics != PYB_SVGD_REFERENCE_LIVE && !fold_prior && !pshard) {
@@ -1364,6 +1406,7 @@ void svgd_step(pyb_handle* h, const int32_t* idx, int64_t B, double* loss_out) {
                                                         lr_t);
       count_launch(h);
       swept = true;
+      h->svgd_stein_used = STEIN_LIVE_CTA;
     }
     if (R == 1 && h->opt_live_fused && !swept) {
       // one cooperative launch for the whole sweep (falls back to the per-particle launches if it cannot be co-resident)
@@ -1378,8 +1421,10 @@ void svgd_step(pyb_handle* h, const int32_t* idx, int64_t B, double* loss_out) {
         PYB_CUDA(cudaLaunchCooperativeKernel((void*)k_live_sweep, dim3(grid), dim3(256), args, 0, h->stream));
         count_launch(h);
         swept = true;
+        h->svgd_stein_used = STEIN_LIVE_COOP;
       }
     }
+    if (!swept) h->svgd_stein_used = STEIN_LIVE_LAUNCHES;
     for (int rr = 0; rr < R && !swept; ++rr) {
       if (rr == sv.rank) {
         for (int i = 0; i < (int)S; ++i) {

@@ -15,14 +15,15 @@ __device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bflo
 }
 
 // src [R, C] fp32 (row stride lds) -> hi/lo [R, C] bf16 (row stride ldd), same orientation
+// center != nullptr: column c is split as src - center[c]
 __global__ void k_split_rows(const float* src, int64_t R, int C, int64_t lds, __nv_bfloat16* hi, __nv_bfloat16* lo,
-                             int64_t ldd) {
+                             int64_t ldd, const float* center = nullptr) {
   const int64_t total = R * C;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     int64_t r = i / C;
     int c = (int)(i - r * C);
     __nv_bfloat16 h, l;
-    split_bf16(src[r * lds + c], h, l);
+    split_bf16(center ? src[r * lds + c] - center[c] : src[r * lds + c], h, l);
     hi[r * ldd + c] = h;
     lo[r * ldd + c] = l;
   }
@@ -30,12 +31,13 @@ __global__ void k_split_rows(const float* src, int64_t R, int C, int64_t lds, __
 // the same for even C, lds, ldd and 8-byte aligned bases (every row then starts 8-byte aligned in src and 4-byte aligned
 // in hi/lo): two elements per thread, 8-byte loads and 4-byte stores
 __global__ void k_split_rows2(const float* __restrict__ src, int64_t R, int C2, int64_t lds, __nv_bfloat16* __restrict__ hi,
-                              __nv_bfloat16* __restrict__ lo, int64_t ldd) {
+                              __nv_bfloat16* __restrict__ lo, int64_t ldd, const float* __restrict__ center = nullptr) {
   const int64_t total = R * C2;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t r = i / C2;
     const int c = 2 * (int)(i - r * C2);
-    const float2 v = *reinterpret_cast<const float2*>(src + r * lds + c);
+    float2 v = *reinterpret_cast<const float2*>(src + r * lds + c);
+    if (center) { v.x -= center[c]; v.y -= center[c + 1]; }
     __nv_bfloat16 h0, l0, h1, l1;
     split_bf16(v.x, h0, l0);
     split_bf16(v.y, h1, l1);

@@ -683,15 +683,16 @@ void tc_forward_tracked(pyb_handle* h, const float* theta, int64_t S, const floa
 }
 
 // ---- building blocks exported to svgd.cu (Gram matrix and Stein contraction on the tensor cores) ----
-void tc_split_rows(pyb_handle* h, const float* src, int64_t R, int C, int64_t lds, void* hi, void* lo, int64_t ldd) {
+void tc_split_rows(pyb_handle* h, const float* src, int64_t R, int C, int64_t lds, void* hi, void* lo, int64_t ldd,
+                   const float* center) {
   const bool pairs = (C % 2 == 0) && (lds % 2 == 0) && (ldd % 2 == 0) && ((uintptr_t)src % 8 == 0) &&
                      ((uintptr_t)hi % 4 == 0) && ((uintptr_t)lo % 4 == 0);
   if (pairs)
     k_split_rows2<<<(unsigned)std::min<int64_t>((R * (C / 2) + 255) / 256, 16 * (int64_t)h->sm_count), 256, 0, h->stream>>>(
-        src, R, C / 2, lds, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, ldd);
+        src, R, C / 2, lds, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, ldd, center);
   else
     k_split_rows<<<(unsigned)std::min<int64_t>((R * C + 255) / 256, 65535), 256, 0, h->stream>>>(
-        src, R, C, lds, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, ldd);
+        src, R, C, lds, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, ldd, center);
   count_launch(h);
 }
 // src [R, C] fp32 -> hi/lo [C, R] bf16 with row pitch ldd

@@ -112,7 +112,10 @@ int pyb_set_option(pyb_handle* h, const char* key, double value);
 /* read-outs: "path_used", "kernel_launches", "last_device_ms", "workspace_bytes", "tensor_path_ok", "hmc_arena_rows"
  * (rows of the device sample arena, 0 while it has never been sized), "fs_cluster_used" (CTAs per chain of the last
  * small-width HMC launch: 1, 2, 4 or 8; 0 before the first), "hmc_param_bytes" (device bytes held by
- * pyb_hmc_track_params) */
+ * pyb_hmc_track_params), "svgd_stein_used" (Stein-update branch of the last pyb_svgd_step or canonical pyb_svgd_phi:
+ * 0 live sweep as per-particle launches, 1 live sweep as one cooperative launch, 2 live sweep in one CTA, 3 canonical on
+ * the float64 kernels, 4 canonical on the tensor cores, 5 canonical on the tensor cores sharded over the parameters;
+ * 0 before the first call; the live-formula pyb_svgd_phi leaves it unchanged) */
 int pyb_get_info(const pyb_handle* h, const char* key, double* value_out);
 
 /* ---- inputs ---- */

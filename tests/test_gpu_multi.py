@@ -106,21 +106,23 @@ def test_predictive_sharded_over_two_gpus_matches_one_gpu():
         np.testing.assert_allclose(r[4], tot, rtol=1e-5, atol=1e-7)
 
 
-def _wide_setup():
+def _wide_setup(offset=0.0):
     rng = np.random.default_rng(11)
     D, H, C, N, B, S, steps = 784, 128, 10, 2048, 512, 512, 3
     X = rng.random((N, D)).astype(np.float32)
     y = rng.integers(0, C, N).astype(np.int32)
     P = D * H + H + H * C + C
     parts = rng.normal(0, 0.05, (S, P))
+    if offset:                  # particles close together around a common point far from the origin
+        parts += offset * np.random.default_rng(12).standard_normal(P)
     idx = [rng.permutation(N)[:B].astype(np.int32) for _ in range(steps)]
     return D, H, C, X, y, parts, idx
 
 
-def _wide_run(rank, world, uid, pshard):
+def _wide_run(rank, world, uid, pshard, offset=0.0):
     from bayesian_inference_for_nn_b200 import _lib, keras_json
     from bayesian_inference_for_nn_b200.engine import Engine
-    D, H, C, X, y, parts, idx = _wide_setup()
+    D, H, C, X, y, parts, idx = _wide_setup(offset)
     S = parts.shape[0]
     Sl = S // world
     eng = Engine(keras_json.parse_model_json(keras_json.make_sequential_json(D, [H, C], ["relu", "softmax"])), device=rank)
@@ -141,26 +143,29 @@ def _wide_run(rank, world, uid, pshard):
     return res
 
 
-def _wide_worker(rank, world, uid, pshard, out):
-    out.put(_wide_run(rank, world, uid, pshard))
+def _wide_worker(rank, world, uid, pshard, offset, out):
+    out.put(_wide_run(rank, world, uid, pshard, offset))
 
 
-@pytest.mark.parametrize("pshard", [1, 2, 0])
-def test_svgd_sharded_on_the_tensor_path_matches_one_gpu(pshard):
+@pytest.mark.parametrize("pshard,offset", [pytest.param(1, 0.0, id="1"), pytest.param(2, 0.0, id="2"), pytest.param(0, 0.0, id="0"),
+                                           pytest.param(1, 1.0, id="1-offset"), pytest.param(0, 1.0, id="0-offset")])
+def test_svgd_sharded_on_the_tensor_path_matches_one_gpu(pshard, offset):
     """C4's shape in small (784-128-10, 512 particles, minibatch 512, canonical median-heuristic update): the sharded step
     on the tensor path — pshard = 1: Stein phase sharded over the parameters, the gradient rows and the updated particle
     blocks exchanged by peer-memory stores of the library's own kernels (CUDA IPC between the rank processes), all-reduced
     Gram matrix and radix-select histograms; 2: the same with NCCL send / recv exchanges; 0: row-sharded with particle and
-    gradient all-gathers — against the SAME step on one GPU: losses, bandwidth h and particles after three steps."""
+    gradient all-gathers — against the SAME step on one GPU: losses, bandwidth h and particles after three steps.
+    offset = 1: the particles sit around a common point far from the origin (each rank centres its own parameter slice
+    with pshard = 1, every rank the same gathered particles with pshard = 0)."""
     from bayesian_inference_for_nn_b200 import _lib
     if _lib.device_count() < 2:
         pytest.skip("needs 2 GPUs")
     import multiprocessing as mp
-    _, one_parts, one_losses, one_h, _ = _wide_run(0, 1, None, 0)
+    _, one_parts, one_losses, one_h, _ = _wide_run(0, 1, None, 0, offset)
     ctx = mp.get_context("spawn")
     uid = _lib.nccl_unique_id()
     q = ctx.Queue()
-    procs = [ctx.Process(target=_wide_worker, args=(r, 2, uid, pshard, q)) for r in range(2)]
+    procs = [ctx.Process(target=_wide_worker, args=(r, 2, uid, pshard, offset, q)) for r in range(2)]
     for p in procs:
         p.start()
     res = sorted([q.get(timeout=300) for _ in range(2)], key=lambda t: t[0])
